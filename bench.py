@@ -12,7 +12,7 @@ arms run all three stages: ours on the device, the reference arm through the com
 ptm_mgau_frame_eval and hmm_vit_eval on the host cores.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                  [--model baseline|en-us] [--utts U] [--secs S]
+                  [--model baseline|en-us] [--utts U] [--secs S] [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for what each key means.
 """
@@ -521,6 +521,41 @@ def run_reference(args, pm, raw, desc, feats, T):
     print(json.dumps(out))
 
 
+def dump_outputs(out_dir, torch, batch, pm, total, H, d_best, d_pen, d_swbest):
+    """Writes what the last timed step left on the device to out_dir/<name>.npy (integers as float64, int16 scores as
+    float32, all exact; under 50 MB in all): the phone loop's best score per frame and the search-scale sweep's best
+    score per (frame, utterance), whole up to 2^20 values; the phone-loop penalties and the senone scores (GBs at the
+    default shape) on a fixed, seeded sample of frames.  A sampled array comes with <name>_rows.npy, the flat indices
+    (rows) it holds.  The inputs are seeded, so two builds run with the same arguments can be compared file by file."""
+    os.makedirs(out_dir, exist_ok=True)
+    dev = torch.device("cuda", torch.cuda.current_device())
+
+    class DeviceArray:                      # a buffer the C API owns, seen by torch without a copy
+        def __init__(self, ptr, shape, typestr):
+            self.__cuda_array_interface__ = {"shape": shape, "typestr": typestr, "data": (ptr, False), "strides": None,
+                                              "version": 3}
+
+    def view(ptr, shape, typestr):
+        return torch.as_tensor(DeviceArray(ptr, shape, typestr), device=dev)
+
+    rng = np.random.default_rng(7)
+
+    def save(name, x, cap, dtype):
+        n = x.shape[0]
+        if n > cap:
+            rows = np.sort(rng.choice(n, cap, replace=False))
+            x = x[torch.from_numpy(rows).to(dev)]
+            np.save(os.path.join(out_dir, name + "_rows.npy"), rows.astype(np.float64))
+        np.save(os.path.join(out_dir, name + ".npy"), x.cpu().numpy().astype(dtype))
+
+    save("phoneloop_best", view(d_best, (total,), "<i4"), 1 << 20, np.float64)
+    save("phoneloop_pen", view(d_pen, (total, H), "<i4"), 4096, np.float64)
+    save("senscr", view(batch.senscr_device_ptr(), (total, pm.n_sen), "<i2"), max(1, (16 << 20) // (4 * pm.n_sen)), np.float32)
+    if d_swbest is not None:
+        sw = d_swbest if d_swbest.numel() <= 1 << 20 else d_swbest.reshape(-1)
+        save("sweep_best", sw, 1 << 20, np.float64)
+
+
 def workload_name(args, pm):
     n = ("%dutt_total" % args.batch_total) if getattr(args, "batch_total", 0) else ("%dutt" % args.utts)
     return "%s_%dx%dx%d_%dsen_%s_x_%ds" % (pm.kind, pm.n_mgau, pm.n_feat, pm.n_density, pm.n_sen, n, args.secs)
@@ -541,7 +576,11 @@ def main():
     ap.add_argument("--cpu-budget", type=float, default=15.0)
     ap.add_argument("--search", default="none", choices=["none", "fwdtree", "fsg"],
                     help="also couple a search kernel to the GMM stage's scores (BASELINE configs 3 / 4), reported as `search_coupled`")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (rank 0's shard) to DIR/<name>.npy, for comparing two builds")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -631,11 +670,13 @@ def main():
     batch.event_record(0)
     kern = {"transpose": 0.0, "topn": 0.0, "senone": 0.0}
     for _ in range(args.steps):
-        batch.decode_device(pl, d_feats.data_ptr(), off)
+        d_best, d_pen = batch.decode_device(pl, d_feats.data_ptr(), off)
         sweep()
     batch.event_record(1)
     ms_total = batch.event_elapsed_ms()
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, torch, batch, pm, total, H, d_best, d_pen, d_swbest if hs is not None else None)
     launches = api.lib().psb_kernel_launch_count() - launches1
     # per-kernel durations for the roofline: two extra steps forced onto ONE stream (with
     # PSB_PIPELINE > 1 the timed region's kernels overlap and cannot be timed individually)

@@ -40,11 +40,11 @@ def test_every_triple_of_the_small_lms(which):
     assert np.array_equal(oracle.lm_scores(arr, q), want)
 
 
-BIG_LM = os.path.join(os.environ.get("PS_REFERENCE", "/root/reference"), "model", "en-us", "en-us.lm.bin")
+BIG_LM = os.path.join(REF, "model", "en-us.lm.bin")
 
 
 @live
-@pytest.mark.skipif(not os.path.exists(BIG_LM), reason="en-us.lm.bin only exists next to the reference sources")
+@pytest.mark.skipif(not os.path.exists(BIG_LM), reason="oracle/_ref/model/en-us.lm.bin not built")
 def test_en_us_lm_existing_ngrams_and_random_queries():
     hd, dic = os.path.join(REF, "model", "en-us"), os.path.join(REF, "model", "cmudict-en-us.dict")
     arr, _ = refdrv.lm_arrays(hd, BIG_LM, dic)

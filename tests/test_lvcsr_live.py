@@ -13,9 +13,9 @@ from test_ngf_emul import emuls, run_second  # noqa: F401
 from test_ngs_emul import run_emul as run_first
 
 REF = os.path.dirname(refdrv.LIB_PATH)
-BIG_LM = os.path.join(os.environ.get("PS_REFERENCE", "/root/reference"), "model", "en-us", "en-us.lm.bin")
+BIG_LM = os.path.join(REF, "model", "en-us.lm.bin")
 pytestmark = [pytest.mark.skipif(not refdrv.available(), reason="oracle/_ref/libpsref.so not built"),
-              pytest.mark.skipif(not os.path.exists(BIG_LM), reason="en-us.lm.bin only exists next to the reference sources")]
+              pytest.mark.skipif(not os.path.exists(BIG_LM), reason="oracle/_ref/model/en-us.lm.bin not built")]
 
 
 def test_large_vocabulary_decode(emuls):  # noqa: F811

@@ -16,9 +16,8 @@ from test_ngs_emul import emul, run_emul  # noqa: F401  (fixture)
 
 pytestmark = pytest.mark.skipif(not refdrv.available(), reason="oracle/_ref/libpsref.so not built")
 REF = os.path.dirname(refdrv.LIB_PATH)
-SRC = os.environ.get("PS_REFERENCE", "/root/reference")
-LM, DIC = os.path.join(SRC, "test/data/turtle.lm.bin"), os.path.join(SRC, "test/data/turtle.dic")
-needs_lm = pytest.mark.skipif(not os.path.exists(LM), reason="turtle LM only exists next to the reference sources")
+LM, DIC = os.path.join(REF, "data", "turtle.lm.bin"), os.path.join(REF, "data", "turtle.dic")
+needs_lm = pytest.mark.skipif(not os.path.exists(LM), reason="oracle/_ref/data/turtle.lm.bin not built")
 HD = os.path.join(REF, "model", "en-us")
 
 

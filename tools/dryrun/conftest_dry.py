@@ -1,10 +1,12 @@
 # Dry run of the gated GPU tests on the CPU: torch's .cuda() becomes the identity and HmmContext's search
 # methods are served by the host emulation harnesses (same argument conventions as the real API).
+# PSB_ROOT: the repository (run.sh copies this file out of it); PSB_EMUL_DIR: where lib{fsg,ngs,ngf}emul.so were built.
 import ctypes as C, os, sys
 import numpy as np
 import pytest
-sys.path.insert(0, "/root/repo"); sys.path.insert(0, "/root/repo/tests")
-exec(open("/root/repo/tests/conftest.py").read().replace("os.path.dirname(os.path.dirname(os.path.abspath(__file__)))", '"/root/repo"'))
+ROOT = os.environ.get("PSB_ROOT") or os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
+exec(open(os.path.join(ROOT, "tests", "conftest.py")).read().replace("os.path.dirname(os.path.dirname(os.path.abspath(__file__)))", repr(ROOT)))
 import torch
 torch.Tensor.cuda = lambda self, *a, **k: self
 _to = torch.Tensor.to
@@ -14,7 +16,7 @@ import test_fsg_emul as TF, test_ngs_emul as TN, test_ngf_emul as TG
 class FakeCtx:
     def __init__(self, tp, sseq, n_sen, device=0):
         self.m = dict(tp=tp, sseq=sseq, phone_tmat=None, phone_ssid=None); self.n_sen = n_sen
-        self.L = {k: C.CDLL("/tmp/lib%semul.so" % k) for k in ("fsg", "ngs", "ngf")}
+        self.L = {k: C.CDLL(os.path.join(os.environ["PSB_EMUL_DIR"], "lib%semul.so" % k)) for k in ("fsg", "ngs", "ngf")}
         self.f_fsg = self.L["fsg"].fsg_emul_run; self.f_fsg.restype = C.c_int32; self.f_fsg.argtypes = TF.ARGT
         self.f1 = self.L["ngs"].ngs_emul_run; self.f1.restype = C.c_int32; self.f1.argtypes = TN.ARGT
         self.f2 = self.L["ngf"].ngf_emul_run; self.f2.restype = C.c_int32; self.f2.argtypes = TG.ARGT

@@ -4,7 +4,8 @@
 # unchanged and must reproduce a plain reference decode (words, score, every segment).  Run by tools/dryrun/run.sh.
 import os, sys, types
 import numpy as np
-sys.path.insert(0, "/root/repo"); sys.path.insert(0, "/root/repo/tools/dryrun")
+HERE = os.path.dirname(os.path.abspath(__file__))
+sys.path.insert(0, os.path.dirname(os.path.dirname(HERE))); sys.path.insert(0, HERE)
 import conftest_dry as D
 from oracle import refdrv
 from pocketsphinx_b200 import api as real_api, decoder

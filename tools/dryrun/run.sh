@@ -7,9 +7,10 @@
 set -e
 ROOT=$(cd "$(dirname "$0")/../.." && pwd)
 D=$(mktemp -d)
+export PSB_ROOT="$ROOT" PSB_EMUL_DIR="$D"
 python -c "from oracle import oracle; oracle.build()" 2>/dev/null || (cd "$ROOT" && python -c "from oracle import oracle; oracle.build()")
 for h in fsg ngs ngf; do
-    g++ -O1 -fPIC -shared -ffp-contract=off -o /tmp/lib${h}emul.so "$ROOT/tests/emul/${h}_emul.cpp" -L"$ROOT/oracle/_build" -lpsoracle -Wl,-rpath,"$ROOT/oracle/_build"
+    g++ -O1 -fPIC -shared -ffp-contract=off -o "$D/lib${h}emul.so" "$ROOT/tests/emul/${h}_emul.cpp" -L"$ROOT/oracle/_build" -lpsoracle -Wl,-rpath,"$ROOT/oracle/_build"
 done
 cp "$ROOT/tools/dryrun/conftest_dry.py" "$D/conftest.py"
 for f in test_gpu_zz_fsg.py test_gpu_zz_ngram.py; do
