@@ -182,7 +182,7 @@ extern "C" int psb_model_create(const psb_model_desc_t *d, int device, psb_model
     m->has_topn_beam = false;
     m->d_topn_beam = nullptr;
     m->tc_ok = false;
-    m->d_tc_wfrag = m->d_tc_wumma = m->d_tc_cen = m->d_tc_bnd = nullptr;
+    m->d_tc_wumma = m->d_tc_cen = m->d_tc_bnd = nullptr;
     m->d_msT = m->d_msdetT = nullptr; m->d_featlen = m->d_featoff = nullptr;
     for (int f = 0; f < PSB_MAX_FEAT; ++f) m->topn_beam[f] = 0;
     const bool dev = d->on_device != 0;
@@ -270,8 +270,6 @@ extern "C" int psb_model_create(const psb_model_desc_t *d, int device, psb_model
             uint8_t t[256];
             if (cudaMemcpy(t, m->d_logadd8, 256, cudaMemcpyDeviceToHost) == cudaSuccess)
                 for (int i = 0; i < 256; ++i) m->logadd8_max = std::max<int>(m->logadd8_max, t[i]);
-                m->logadd8_zero_from = 256;
-                while (m->logadd8_zero_from > 0 && t[m->logadd8_zero_from - 1] == 0) --m->logadd8_zero_from;
         }
     }
     if (!rc && m->kind != PSB_KIND_MS && !d->logadd8) {
@@ -312,7 +310,7 @@ extern "C" void psb_model_free(psb_model_t *m)
     cudaFree(m->d_rec); cudaFree(m->d_rec_off); cudaFree(m->d_rec2); cudaFree(m->d_rec2_off); cudaFree(m->d_mixw); cudaFree(m->d_mixw_cb);
     cudaFree(m->d_sen2cb); cudaFree(m->d_sen2cb32); cudaFree(m->d_quadcb); cudaFree(m->d_bsen); cudaFree(m->d_logadd8); cudaFree(m->d_logadd_ms);
     cudaFree(m->d_topn_beam); cudaFree(m->d_msT); cudaFree(m->d_msdetT); cudaFree(m->d_featlen); cudaFree(m->d_featoff);
-    cudaFree(m->d_tc_wfrag); cudaFree(m->d_tc_wumma); cudaFree(m->d_tc_cen); cudaFree(m->d_tc_bnd);
+    cudaFree(m->d_tc_wumma); cudaFree(m->d_tc_cen); cudaFree(m->d_tc_bnd);
     delete m;
 }
 
@@ -339,10 +337,15 @@ extern "C" int psb_batch_create(psb_model_t *m, int32_t max_utts, int64_t max_fr
     b->max_utts = max_utts;
     b->max_frames = max_frames;
     {
-        // tuning knob; default = tensor-core filter + exact rescoring (psb_ptm_tc.cu) where the model allows it,
-        // else packed FP32 with deferred insertion (ptm_topnq_kernel, variant 5)
+        // 6 (default): tensor-core filter + exact rescoring (psb_ptm_tc.cu) where the model allows it, else the scan
+        // kernels (psb_ptm.cu); 5: the scan kernels everywhere, the reference the filter is tested against
         const char *v = getenv("PSB_TOPN_VARIANT");
-        b->topn_variant = v ? atoi(v) : 6;
+        if (v && strcmp(v, "5") && strcmp(v, "6")) {
+            psb_set_error("psb_batch_create: PSB_TOPN_VARIANT=%s is not supported (accepted: 5 = scan kernels, 6 = default)", v);
+            delete b;
+            return PSB_ERR_ARG;
+        }
+        b->force_scan = v && !strcmp(v, "5");
         const char *p = getenv("PSB_PIPELINE");         // sub-batches in flight for psb_decode_batch_*
         b->n_pipe = p ? atoi(p) : 0;                   // 0 = auto (see decode_common)
         if (b->n_pipe < 0) b->n_pipe = 0;
@@ -503,7 +506,7 @@ static int get_kid(psb_batch_t *b, int i, psb_batch_t **out)
 {
     while ((int)b->kids.size() <= i) {
         psb_batch_t *k = new psb_batch_t();
-        k->m = b->m; k->max_utts = b->max_utts; k->max_frames = b->max_frames; k->topn_variant = b->topn_variant;
+        k->m = b->m; k->max_utts = b->max_utts; k->max_frames = b->max_frames; k->force_scan = b->force_scan;
         k->is_kid = true; k->n_pipe = 1;
         cudaError_t e = cudaStreamCreateWithFlags(&k->stream, cudaStreamNonBlocking);
         for (int j = 0; j < 4 && e == cudaSuccess; ++j) e = cudaEventCreate(&k->ev[j]);

@@ -526,7 +526,7 @@ extern "C" int psb_phoneloop_run_host(psb_phoneloop_t *p, const int16_t *senscr,
 // never reach the best score.
 constexpr int HS_V = 4;                     // instances per thread
 constexpr int HS_TS = 512;                  // storage tile: [tile][field][HS_TS], so a CTA's fields are one contiguous block
-// threads per CTA: 128 (default; measured 112.7 us vs 118.2 us per 6.08 M-instance frame) or 256 (PSB_HMMSET_THREADS)
+constexpr int HS_THREADS = 128;             // threads per CTA of hmmset_eval_kernel: 112.7 us against 118.2 us at 256 per 6.08 M-instance frame
 
 struct psb_hmmset_s {
     psb_hmmctx_t *c;
@@ -652,7 +652,7 @@ __device__ __forceinline__ void tma_bulk_g2s(void *dst, const void *src, unsigne
 // segment.  row0[seg] + t is the segment's senone-score row of this frame (staged in shared
 // memory: the gathers of a tile hit ~3 x HS_TILE random int16 of it); segments with
 // n_rows[seg] <= t are finished.  NS = 3 or 5 (0: any topology, runtime count).
-template <int NS, int HS_THREADS>
+template <int NS>
 __global__ void __launch_bounds__(HS_THREADS, (NS == 3 ? 3 : 2) * (256 / HS_THREADS))
 hmmset_eval_kernel(HmmSetDev s, HmmCtxDev c, const int16_t *__restrict__ senscr, const int64_t *__restrict__ row0,
                    const int32_t *__restrict__ n_rows, int t, int32_t *__restrict__ best_out)
@@ -1229,37 +1229,26 @@ extern "C" int psb_hmmset_eval_frames_device(psb_hmmset_t *s, const int16_t *d_s
         PSB_CUDA(cudaStreamSynchronize(s->stream));
         return PSB_OK;
     }
-    static const int threads = [] {
-        const char *v = getenv("PSB_HMMSET_THREADS");
-        return v && atoi(v) == 256 ? 256 : 128;
-    }();
-    const int tile = threads * HS_V;
+    const int tile = HS_THREADS * HS_V;
     const dim3 grid((unsigned)((s->max_seg_len + tile - 1) / tile), (unsigned)s->n_seg);
     const HmmSetDev sd = dev_set(s);
     const HmmCtxDev cd = dev_ctx(s->c);
     const size_t smem = (((size_t)cd.n_sen * 2 + 15) & ~(size_t)15) + 16;      // the row keeps its alignment within 16 bytes
     PSB_REQUIRE(smem <= 200 * 1024, "psb_hmmset: %d senones do not fit the shared-memory score row", cd.n_sen);
     auto launch = [&](auto kern, int t, int32_t *best) {
-        kern<<<grid, threads, smem, s->stream>>>(sd, cd, d_senscr, d_row0, d_n_rows, t, best);
+        kern<<<grid, HS_THREADS, smem, s->stream>>>(sd, cd, d_senscr, d_row0, d_n_rows, t, best);
     };
-#define PSB_HS_ATTR(NS, NT) PSB_CUDA(cudaFuncSetAttribute(hmmset_eval_kernel<NS, NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem))
+#define PSB_HS_ATTR(NS) PSB_CUDA(cudaFuncSetAttribute(hmmset_eval_kernel<NS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem))
     if (smem > 48 * 1024) {
-        PSB_HS_ATTR(3, 256); PSB_HS_ATTR(5, 256); PSB_HS_ATTR(0, 256); PSB_HS_ATTR(3, 128); PSB_HS_ATTR(5, 128); PSB_HS_ATTR(0, 128);
+        PSB_HS_ATTR(3); PSB_HS_ATTR(5); PSB_HS_ATTR(0);
     }
 #undef PSB_HS_ATTR
     PSB_CUDA(cudaEventRecord(s->ev[0], s->stream));
     for (int t = 0; t < n_frames; ++t) {
         int32_t *best = d_best + (size_t)t * s->n_seg;
-        if (threads == 256) {
-            if (cd.n_emit == 3) launch(hmmset_eval_kernel<3, 256>, t, best);
-            else if (cd.n_emit == 5) launch(hmmset_eval_kernel<5, 256>, t, best);
-            else launch(hmmset_eval_kernel<0, 256>, t, best);
-        }
-        else {
-            if (cd.n_emit == 3) launch(hmmset_eval_kernel<3, 128>, t, best);
-            else if (cd.n_emit == 5) launch(hmmset_eval_kernel<5, 128>, t, best);
-            else launch(hmmset_eval_kernel<0, 128>, t, best);
-        }
+        if (cd.n_emit == 3) launch(hmmset_eval_kernel<3>, t, best);
+        else if (cd.n_emit == 5) launch(hmmset_eval_kernel<5>, t, best);
+        else launch(hmmset_eval_kernel<0>, t, best);
         PSB_LAUNCH_CHECK();
     }
     PSB_CUDA(cudaEventRecord(s->ev[1], s->stream));
@@ -1285,8 +1274,6 @@ extern "C" int psb_hmmset_sweep_device(psb_hmmset_t *s, const int16_t *d_senscr,
         if (ms) PSB_CUDA(cudaStreamSynchronize(s->stream));
         return PSB_OK;
     }
-    // CTA shape: threads x instances per thread (PSB_SWEEP_SHAPE = 0: 256 x 4 (default), 1: 256 x 2, 2: 128 x 4, 3: 512 x 2)
-    static const int shape = [] { const char *v = getenv("PSB_SWEEP_SHAPE"); return v ? atoi(v) : 0; }();
     const int buf_bytes = (int)(((size_t)cd.n_sen * 2 + 32 + 127) & ~(size_t)127);
     const int tp_bytes = s->c->n_tmat * cd.n_emit * (cd.n_emit + 1);
     const size_t smem = 2 * (size_t)buf_bytes + tp_bytes;
@@ -1301,14 +1288,9 @@ extern "C" int psb_hmmset_sweep_device(psb_hmmset_t *s, const int16_t *d_senscr,
         kern<<<grid, THREADS, smem, s->stream>>>(sd, cd, d_senscr, (long long)rows_total, d_row0, d_n_rows, n_frames, d_best,  \
                                                 s->c->n_tmat, buf_bytes, 0, 0, -1, nullptr);                                   \
     } while (0)
-    if (cd.n_emit == 3) {
-        if (shape == 1) PSB_SWEEP(3, 2, 256);
-        else if (shape == 2) PSB_SWEEP(3, 4, 128);
-        else if (shape == 3) PSB_SWEEP(3, 2, 512);
-        else PSB_SWEEP(3, 4, 256);
-    }
-    else
-        PSB_SWEEP(5, 4, 256);
+    // CTA shape: 256 threads x 4 instances per thread
+    if (cd.n_emit == 3) PSB_SWEEP(3, 4, 256);
+    else PSB_SWEEP(5, 4, 256);
 #undef PSB_SWEEP
     PSB_LAUNCH_CHECK();
     PSB_CUDA(cudaEventRecord(s->ev[1], s->stream));
@@ -1415,8 +1397,8 @@ extern "C" int psb_hmmset_eval_host(psb_hmmset_t *s, const int16_t *senscr, int3
 // its evaluate_hmms, state_align_search.c:65).  One CTA per utterance, the utterance's phone
 // chain in shared memory (SoA), time is the loop inside the kernel: renormalise (:199-203),
 // evaluate_hmms (:64-86), prune_hmms (:88-107), phone_transition (:109-136, a left-to-right
-// scan whose hmm_enter can cascade through not-yet-active successors, so one thread walks it in
-// the reference's order), record_transitions (:153-182) into a token table in HBM, and at the end
+// scan whose hmm_enter can cascade through not-yet-active successors: one warp resolves it as a
+// carry chain, see below), record_transitions (:153-182) into a token table in HBM, and at the end
 // the backtrace of state_align_search_finish (:221-279).
 namespace {
 
@@ -1426,7 +1408,7 @@ align_kernel(const int16_t *__restrict__ senscr, const int32_t *__restrict__ utt
              const int32_t *__restrict__ tmatid_g, const int32_t *__restrict__ sf_g, const int32_t *__restrict__ ef_g,
              int32_t *__restrict__ tok_id, int32_t *__restrict__ tok_sc, const int64_t *__restrict__ tok_off,
              int32_t *__restrict__ st_start, int32_t *__restrict__ st_dur, int32_t *__restrict__ st_score,
-             int32_t *__restrict__ status, bool seq_scan)
+             int32_t *__restrict__ status)
 {
     extern __shared__ int sm[];
     const int u = blockIdx.x, tid = threadIdx.x, N = c.n_emit;
@@ -1498,18 +1480,7 @@ align_kernel(const int16_t *__restrict__ senscr, const int32_t *__restrict__ utt
         // (G reads nothing an earlier iteration writes), "active" is A[i] = P[i] | (G[i] & A[i-1]):
         // a carry chain.  One warp resolves 32 phones per step with a 64-bit add
         // (generate = P, propagate = G & ~P), the carry links the steps; E[j] = A[j-1] & G[j].
-        if (seq_scan) {
-            if (tid == 0)
-                for (int i = 0; i < H - 1; ++i) {
-                    if (frame[i] != nf) continue;
-                    if (nf < (sf_g ? sf_g[p0 + i + 1] : 0)) continue;
-                    const int nps = out_score[i];
-                    if (frame[i + 1] < t || nps > score[i + 1]) {        // hmm_enter(nhmm, score, history, nf)
-                        score[i + 1] = nps; hist[i + 1] = out_hist[i]; frame[i + 1] = nf;
-                    }
-                }
-        }
-        else if (tid < 32) {
+        if (tid < 32) {
             unsigned carry = 0u;
             for (int base = 0; base < H; base += 32) {
                 const int j = base + tid;
@@ -1645,7 +1616,7 @@ extern "C" int psb_align_batch_device(psb_hmmctx_t *c, const int16_t *d_senscr, 
         align_kernel<<<(unsigned)n_utt, 128, smem, st>>>(d_senscr, d_i32 + o_utt, dev_ctx(c), d_i32 + o_ph, c->d_al_senid, d_i32 + o_tm,
                                                         sf ? d_i32 + o_sf : nullptr, ef ? d_i32 + o_ef : nullptr, d_tok,
                                                         d_tok + tok_off[(size_t)n_utt], c->d_al_tokoff, d_i32 + o_ss, d_i32 + o_sd,
-                                                        d_i32 + o_sc, d_i32 + o_st, getenv("PSB_ALIGN_SEQ_SCAN") != nullptr);
+                                                        d_i32 + o_sc, d_i32 + o_st);
         g_psb_launches.fetch_add(1, std::memory_order_relaxed);
         e = cudaGetLastError();
     }

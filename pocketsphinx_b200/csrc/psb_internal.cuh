@@ -81,7 +81,6 @@ struct psb_model_s {
     int32_t *d_bsen;              // senones of the non-uniform quads
     int n_bsen;
     int logadd8_max;              // largest entry of the 8-bit add table (bias bound of the 16x2 senone kernel)
-    int logadd8_zero_from;        // smallest i with table[j] == 0 for all j >= i (<= 31: the two-index table of the senone kernel applies)
     uint8_t *d_logadd8;           // [PSB_LOGADD8_N]: the 256-entry table continued with zeros
     uint32_t *d_logadd_ms;
     float *d_msT, *d_msdetT;      // ms back-end: codebook-minor Gaussians (see psb_ms.cu)
@@ -89,9 +88,9 @@ struct psb_model_s {
     uint8_t topn_beam[PSB_MAX_FEAT];
     int32_t *d_topn_beam;         // [PSB_MAX_FEAT]
     bool has_topn_beam;
-    // tensor-core filter path (psb_ptm_tc.cu): W in mma fragment order, centres, error-bound coefficients
+    // tensor-core filter path (psb_ptm_tc.cu): W in the tcgen05 operand layout, centres, error-bound coefficients
     bool tc_ok;
-    float *d_tc_wfrag, *d_tc_wumma, *d_tc_cen, *d_tc_bnd;
+    float *d_tc_wumma, *d_tc_cen, *d_tc_bnd;
 };
 
 struct psb_batch_s {
@@ -117,9 +116,8 @@ struct psb_batch_s {
     long long last_frames;
     float2 *d_semi_dist; size_t semi_cap;      // semi-continuous split path: {d, partial} per (stream, frame, codeword)
     int32_t *d_uttoff; size_t uttoff_cap;
-    int topn_variant;             // PSB_TOPN_VARIANT: 0 scalar, 1/2 packed FP32, 3 two utterances per lane,
-                                  // 4/5 packed + deferred insertion (2 / 1 utterances per lane),
-                                  // 6 (default) tensor-core filter + exact rescoring where the model allows, else 5
+    bool force_scan;              // PSB_TOPN_VARIANT=5: the scan kernels even where the tensor-core filter applies
+                                  // (6, the default: the model's shape decides)
     unsigned *d_tc_flags; size_t tc_flag_cap, tc_flag_words;   // [K][words]: frames the tie fix-up redoes
     float *d_tc_check;            // debug (PSB_TC_CHECK=1): max |a - d| / eps, max candidates
     uint4 *d_tc_items; unsigned *d_tc_nitems; unsigned tc_item_cap;   // rows the filter left in doubt (ptm_tc_exact_kernel)

@@ -10,8 +10,6 @@
 // L2 traffic by FT.
 #include "psb_internal.cuh"
 
-#include <stdlib.h>
-
 #include <algorithm>
 
 namespace {
@@ -115,11 +113,12 @@ __device__ __forceinline__ int logadd_wide(const uint32_t *__restrict__ tab, int
 // staged transposed ([dimension][frame]), so that one warp-uniform LDS.128 pair feeds eight frames.
 // Per (density, dimension): 2 LDS + 2 broadcast LDS.128 for 32 floating-point operations.  Same
 // arithmetic, same order, same insertion rule as ms_dist_kernel: bit-identical lists.
-// TFT = frames per thread: 8 (eight warps per CTA, 127 registers, 16 warps per SM) or 4 (sixteen warps per CTA at 64
-// registers, 32 warps per SM: twice the shared-memory instructions per floating-point operation, twice the warps to hide them).
-constexpr int MS_TCB = 32, MS_TFB = 64;      // codebooks per CTA, frames per block
+// MS_TFT = 4 frames per thread: sixteen warps per CTA at 64 registers, 32 warps per SM -- against eight frames per
+// thread (127 registers, 16 warps per SM), twice the shared-memory instructions per floating-point operation and twice
+// the warps to hide them.
+constexpr int MS_TCB = 32, MS_TFB = 64, MS_TFT = 4;      // codebooks per CTA, frames per block, frames per thread
 
-// PK: frame PAIRS through FADD2 / FMUL2 (x - m == x + (-m) exactly, the means are staged negated; every product and
+// Frame PAIRS go through FADD2 / FMUL2 (x - m == x + (-m) exactly, the means are staged negated; every product and
 // difference is rounded separately as before and the running sums stay scalar -- ptxas would contract a packed
 // multiply-add): 3 packed + 2 scalar instructions per pair and (density, dimension) instead of 8 scalar.
 // FUSE (continuous models: senone s owns codebook s): the lane that holds a codebook's list evaluates the senone on the spot --
@@ -129,7 +128,7 @@ struct MsSenArgs {
     const uint8_t *pdf; const uint32_t *tab; int tab_size, tab_zero; int16_t *senscr; int32_t *best; int n_used, aw;
 };
 
-template <int NT, int MS_TFT, bool PK, bool FUSE>
+template <int NT, bool FUSE>
 __global__ void __launch_bounds__(MS_TFB / MS_TFT * 32, 2)
 ms_dist_tile_kernel(const float *__restrict__ gT, const float *__restrict__ detT, const float *__restrict__ feats,
                     int2 *__restrict__ out, long long frame0, long long n_frames, int n_mgau, int n_feat, int nd,
@@ -146,14 +145,14 @@ ms_dist_tile_kernel(const float *__restrict__ gT, const float *__restrict__ detT
     const int cbr = cb < n_mgau ? cb : n_mgau - 1;      // padding lanes read the last codebook and write nothing
     for (int r = warp; r < n_rows; r += MS_TFB / MS_TFT) {
         const float g = gT[(size_t)r * n_mgau + cbr];
-        par[r * MS_TCB + lane] = (PK && !(r & 1)) ? -g : g;      // rows alternate mean, variance term
+        par[r * MS_TCB + lane] = !(r & 1) ? -g : g;             // rows alternate mean, variance term
     }
     for (int r = warp; r < n_det; r += MS_TFB / MS_TFT) dets[r * MS_TCB + lane] = detT[(size_t)r * n_mgau + cbr];
     const bool all = NT >= nd;                          // compute_dist_all (ms_gauden.c:378-419)
     const long long f_begin = (long long)blockIdx.y * frames_per_cta;
     const long long f_end = f_begin + frames_per_cta < n_frames ? f_begin + frames_per_cta : n_frames;
     // the next block's features travel while this block is computed: each thread keeps its share in registers
-    constexpr int PRE = MS_TFT == 4 ? 6 : 12, NTHR = MS_TFB / MS_TFT * 32;
+    constexpr int PRE = 6, NTHR = MS_TFB / MS_TFT * 32;
     const bool prefetch = sumlen * MS_TFB <= PRE * NTHR;            // uniform; longer vectors are staged in place
     float pre[PRE];
     auto fetch = [&](long long fb) {
@@ -209,23 +208,14 @@ ms_dist_tile_kernel(const float *__restrict__ gT, const float *__restrict__ detT
                         const float4 xq = *reinterpret_cast<const float4 *>(xp + q);
                         xv[q] = xq.x; xv[q + 1] = xq.y; xv[q + 2] = xq.z; xv[q + 3] = xq.w;
                     }
-                    if (PK) {
-                        const float2 nm2 = make_float2(m, m), vv = make_float2(v, v);        // m holds the negated mean
+                    const float2 nm2 = make_float2(m, m), vv = make_float2(v, v);            // m holds the negated mean
 #pragma unroll
-                        for (int q = 0; q < MS_TFT; q += 2) {
-                            float2 t = __fadd2_rn(make_float2(xv[q], xv[q + 1]), nm2);
-                            t = __fmul2_rn(t, t);
-                            t = __fmul2_rn(t, vv);
-                            dv[q] = __fsub_rn(dv[q], t.x);                                   // :467-470
-                            dv[q + 1] = __fsub_rn(dv[q + 1], t.y);
-                        }
-                    }
-                    else {
-#pragma unroll
-                        for (int q = 0; q < MS_TFT; ++q) {
-                            const float diff = __fsub_rn(xv[q], m);
-                            dv[q] = __fsub_rn(dv[q], __fmul_rn(__fmul_rn(diff, diff), v));   // :467-470
-                        }
+                    for (int q = 0; q < MS_TFT; q += 2) {
+                        float2 t = __fadd2_rn(make_float2(xv[q], xv[q + 1]), nm2);
+                        t = __fmul2_rn(t, t);
+                        t = __fmul2_rn(t, vv);
+                        dv[q] = __fsub_rn(dv[q], t.x);                                       // :467-470
+                        dv[q + 1] = __fsub_rn(dv[q + 1], t.y);
                     }
                 }
 #pragma unroll
@@ -295,91 +285,6 @@ ms_dist_tile_kernel(const float *__restrict__ gT, const float *__restrict__ detT
     }
 }
 
-// EXPERIMENT (PSB_MS_PACKED=1; bit-identical -- the whole GPU suite passes with it -- but measured
-// slightly SLOWER on B200: 181 ms vs 174 ms, the kernel is not issue-bound).
-// Packed-FP32 variant of ms_dist_kernel: the FT = 4 frames of a thread go through FADD2 / FMUL2 two
-// at a time (features staged as float2 pairs, the mean and variance term are scalar-broadcast
-// operands); x - m == x + (-m) exactly, every product and difference is rounded separately and the
-// running sums stay scalar (ptxas would contract a packed multiply-add).  Same bits, fewer issue
-// slots: 2 LDG + 2 LDS.64 + 1 negate + 6 packed + 4 scalar per (density, dimension) instead of
-// 2 LDG + 4 LDS + 16 scalar.
-template <int NT>
-__global__ void __launch_bounds__(128)
-ms_dist2_kernel(const float *__restrict__ gT, const float *__restrict__ detT, const float *__restrict__ feats,
-               int2 *__restrict__ out, long long frame0, long long n_frames, int n_mgau, int n_feat, int nd,
-               int sumlen, const int32_t *__restrict__ featlen, const int32_t *__restrict__ featoff)
-{
-    extern __shared__ float sx[];                     // [FT / 2][sumlen][2]: frame pairs interleaved
-    const long long fbase = (long long)blockIdx.y * FT;
-    for (int i = threadIdx.x; i < FT * sumlen; i += blockDim.x) {
-        const int q = i / sumlen, j = i % sumlen;
-        const long long fr = fbase + q;
-        sx[((q >> 1) * sumlen + j) * 2 + (q & 1)] = fr < n_frames ? feats[(frame0 + fr) * sumlen + j] : 0.f;
-    }
-    __syncthreads();
-    const float2 *sx2 = reinterpret_cast<const float2 *>(sx);
-    const int cb = blockIdx.x * blockDim.x + threadIdx.x;
-    if (cb >= n_mgau) return;
-    const bool all = NT >= nd;                        // compute_dist_all (ms_gauden.c:378-419)
-    for (int f = 0; f < n_feat; ++f) {
-        const int fl = featlen[f], fo = featoff[f];
-        int id[FT][NT];
-        float ds[FT][NT];
-#pragma unroll
-        for (int q = 0; q < FT; ++q)
-#pragma unroll
-            for (int i = 0; i < NT; ++i) { id[q][i] = 0; ds[q][i] = (float)INT_MIN; }     // WORST_DIST (:447-448)
-        const float *gp = gT + ((size_t)fo * nd * 2) * n_mgau + cb;
-        for (int d = 0; d < nd; ++d) {
-            float dv[FT];
-            const float det = detT[((size_t)f * nd + d) * n_mgau + cb];
-#pragma unroll
-            for (int q = 0; q < FT; ++q) dv[q] = det;
-            for (int j = 0; j < fl; ++j) {
-                const float m = gp[((size_t)(d * fl + j) * 2) * n_mgau];
-                const float v = gp[((size_t)(d * fl + j) * 2 + 1) * n_mgau];
-                const float2 nm = make_float2(-m, -m), vv = make_float2(v, v);
-#pragma unroll
-                for (int q = 0; q < FT; q += 2) {
-                    float2 t = __fadd2_rn(sx2[(q >> 1) * sumlen + fo + j], nm);
-                    t = __fmul2_rn(t, t);
-                    t = __fmul2_rn(t, vv);
-                    dv[q] = __fsub_rn(dv[q], t.x);                                        // :467-470
-                    dv[q + 1] = __fsub_rn(dv[q + 1], t.y);
-                }
-            }
-#pragma unroll
-            for (int q = 0; q < FT; ++q) {
-                if (all) {
-#pragma unroll
-                    for (int i = 0; i < NT; ++i)
-                        if (i == d) { id[q][i] = d; ds[q][i] = dv[q]; }
-                }
-                else if (dv[q] >= ds[q][NT - 1]) {     // early exit is result-neutral (:457,:474)
-                    // insert before the first entry that is not better (strict '<' scan, :478-483)
-                    int p = 0;
-#pragma unroll
-                    for (int i = 0; i < NT; ++i) p += (dv[q] < ds[q][i]) ? 1 : 0;
-#pragma unroll
-                    for (int i = NT - 1; i > 0; --i)
-                        if (i > p) { ds[q][i] = ds[q][i - 1]; id[q][i] = id[q][i - 1]; }
-#pragma unroll
-                    for (int i = 0; i < NT; ++i)
-                        if (i == p) { ds[q][i] = dv[q]; id[q][i] = d; }
-                }
-            }
-        }
-#pragma unroll
-        for (int q = 0; q < FT; ++q) {
-            const long long fr = fbase + q;
-            if (fr >= n_frames) break;
-            int2 *o = out + ((fr * n_mgau + cb) * n_feat + f) * NT;
-#pragma unroll
-            for (int i = 0; i < NT; ++i) o[i] = make_int2(id[q][i], __float_as_int(ds[q][i]));
-        }
-    }
-}
-
 // senone_eval (ms_senone.c:358-407) + the first clamp; raw scores and the per-frame minimum.
 __global__ void __launch_bounds__(256)
 ms_senone_kernel(const int2 *__restrict__ dist, const uint8_t *__restrict__ pdf, const int32_t *__restrict__ sen2cb,
@@ -440,109 +345,7 @@ __global__ void fill_i32(int32_t *p, long long n, int32_t v)
     if (i < n) p[i] = v;
 }
 
-
-// EXPERIMENT (PSB_MS_REGTILE=1; bit-identical, but measured SLOWER on B200: 247 ms vs 174 ms for
-// 255 k frames of the 5138 x 8 x 39 model, so it is off by default).
-// Register-tiled variant for small codebooks (n_density <= ND_MAX, the continuous-model case):
-// ms_dist_kernel issues one shared-memory load per 4 flops (the feature value of each frame for
-// every (density, dimension)); here a chunk of CH dimensions of the FT frames sits in registers
-// while ALL densities stream past it, so per 4 * FT flops there are two coalesced parameter loads
-// and no feature load.  Every (frame, density) sum still adds its dimensions in ascending order
-// and the top-N insertion runs over the densities in order afterwards: same bits.
-constexpr int ND_MAX = 8;
-constexpr int CH = 13;
-template <int NT>
-__global__ void __launch_bounds__(128)
-ms_dist_reg_kernel(const float *__restrict__ gT, const float *__restrict__ detT, const float *__restrict__ feats,
-                   int2 *__restrict__ out, long long frame0, long long n_frames, int n_mgau, int n_feat, int nd,
-                   int sumlen, const int32_t *__restrict__ featlen, const int32_t *__restrict__ featoff)
-{
-    extern __shared__ float sx[];                     // [FT][sumlen]
-    const long long fbase = (long long)blockIdx.y * FT;
-    for (int i = threadIdx.x; i < FT * sumlen; i += blockDim.x) {
-        const long long fr = fbase + i / sumlen;
-        sx[i] = fr < n_frames ? feats[(frame0 + fr) * sumlen + i % sumlen] : 0.f;
-    }
-    __syncthreads();
-    const int cb = blockIdx.x * blockDim.x + threadIdx.x;
-    if (cb >= n_mgau) return;
-    const bool all = NT >= nd;
-    for (int f = 0; f < n_feat; ++f) {
-        const int fl = featlen[f], fo = featoff[f];
-        const float *gp = gT + ((size_t)fo * nd * 2) * n_mgau + cb;
-        float dv[FT][ND_MAX];
-#pragma unroll
-        for (int d = 0; d < ND_MAX; ++d) {
-            const float det = d < nd ? detT[((size_t)f * nd + d) * n_mgau + cb] : 0.f;
-#pragma unroll
-            for (int q = 0; q < FT; ++q) dv[q][d] = det;
-        }
-        for (int j0 = 0; j0 < fl; j0 += CH) {
-            float x[FT][CH];
-#pragma unroll
-            for (int q = 0; q < FT; ++q)
-#pragma unroll
-                for (int jj = 0; jj < CH; ++jj) x[q][jj] = j0 + jj < fl ? sx[q * sumlen + fo + j0 + jj] : 0.f;
-#pragma unroll
-            for (int d = 0; d < ND_MAX; ++d) {
-                if (d >= nd) break;
-#pragma unroll
-                for (int jj = 0; jj < CH; ++jj) {
-                    if (j0 + jj >= fl) break;
-                    const float m = gp[((size_t)(d * fl + j0 + jj) * 2) * n_mgau];
-                    const float v = gp[((size_t)(d * fl + j0 + jj) * 2 + 1) * n_mgau];
-#pragma unroll
-                    for (int q = 0; q < FT; ++q) {
-                        const float diff = __fsub_rn(x[q][jj], m);
-                        dv[q][d] = __fsub_rn(dv[q][d], __fmul_rn(__fmul_rn(diff, diff), v));
-                    }
-                }
-            }
-        }
-        int id[FT][NT];
-        float ds[FT][NT];
-#pragma unroll
-        for (int q = 0; q < FT; ++q)
-#pragma unroll
-            for (int i = 0; i < NT; ++i) { id[q][i] = 0; ds[q][i] = (float)INT_MIN; }
-#pragma unroll
-        for (int d = 0; d < ND_MAX; ++d) {
-            if (d >= nd) break;
-#pragma unroll
-            for (int q = 0; q < FT; ++q) {
-                const float val = dv[q][d];
-                if (all) {
-#pragma unroll
-                    for (int i = 0; i < NT; ++i)
-                        if (i == d) { id[q][i] = d; ds[q][i] = val; }
-                }
-                else if (val >= ds[q][NT - 1]) {
-                    int p = 0;
-#pragma unroll
-                    for (int i = 0; i < NT; ++i) p += (val < ds[q][i]) ? 1 : 0;
-#pragma unroll
-                    for (int i = NT - 1; i > 0; --i)
-                        if (i > p) { ds[q][i] = ds[q][i - 1]; id[q][i] = id[q][i - 1]; }
-#pragma unroll
-                    for (int i = 0; i < NT; ++i)
-                        if (i == p) { ds[q][i] = val; id[q][i] = d; }
-                }
-            }
-        }
-#pragma unroll
-        for (int q = 0; q < FT; ++q) {
-            const long long fr = fbase + q;
-            if (fr >= n_frames) break;
-            int2 *o = out + ((fr * n_mgau + cb) * n_feat + f) * NT;
-#pragma unroll
-            for (int i = 0; i < NT; ++i) o[i] = make_int2(id[q][i], __float_as_int(ds[q][i]));
-        }
-    }
-}
-
 }  // namespace
-
-static bool reg_tile_env() { static const bool v = getenv("PSB_MS_REGTILE") != nullptr; return v; }
 
 int psb_launch_ms_batch(psb_batch_t *b, const float *d_feats, const int32_t *utt_off, int32_t n_utt, int16_t *d_senscr)
 {
@@ -574,44 +377,31 @@ int psb_launch_ms_batch(psb_batch_t *b, const float *d_feats, const int32_t *utt
         dim3 g1((m->n_mgau + 127) / 128, (unsigned)((n + FT - 1) / FT));
         size_t smem = (size_t)FT * m->sumlen * sizeof(float);
         int2 *dist = reinterpret_cast<int2 *>(b->d_msdist);
-        static const bool packed = getenv("PSB_MS_PACKED") != nullptr;       // experiment, off: bit-identical, 181 vs 174 ms
-        static const bool no_tile = getenv("PSB_MS_NOTILE") != nullptr;     // PSB_MS_NOTILE=1: the round-1 kernel (parameters streamed from L2)
+        // the Gaussians of a 32-codebook tile in shared memory when they fit, else ms_dist_kernel (parameters from L2)
         const size_t tile_smem = ((size_t)m->n_density * m->sumlen * 2 + (size_t)m->n_feat * m->n_density) * MS_TCB * sizeof(float)
                                  + (size_t)m->sumlen * MS_TFB * sizeof(float);
-        const bool tile = !no_tile && !packed && !reg_tile_env() && tile_smem <= 100 * 1024;
-        static const bool tile_tft4 = [] { const char *v = getenv("PSB_MS_TFT"); return !(v && atoi(v) == 8); }();   // frames per thread: 4 (default) or 8
-        static const bool tile_pk = [] { const char *v = getenv("PSB_MS_PK"); return !(v && atoi(v) == 0); }();       // packed FP32 pairs (default) or scalar
+        const bool tile = tile_smem <= 100 * 1024;
         // frames per CTA: enough CTAs for ~4 waves of two resident CTAs per SM, whole 32-frame blocks
         const int tiles_x = (m->n_mgau + MS_TCB - 1) / MS_TCB;
         long long fpc = (n * tiles_x + 148LL * 2 * 4 - 1) / (148LL * 2 * 4);
         fpc = std::max<long long>(MS_TFB, (fpc + MS_TFB - 1) / MS_TFB * MS_TFB);
         const dim3 gt((unsigned)tiles_x, (unsigned)((n + fpc - 1) / fpc));
-        static const bool reg_tile = getenv("PSB_MS_REGTILE") != nullptr;   // experiment, off: measured slower (247 vs 174 ms)
-        static const bool no_fuse = [] { const char *v = getenv("PSB_MS_FUSE"); return v && atoi(v) == 0; }();
         // continuous models: mixtures evaluated by the lane that holds the list (the kernel writes raw scores and minima)
-        const bool fuse = tile && !no_fuse && m->sen_is_cb && tile_tft4 && tile_pk && m->n_mgau > 1;
+        const bool fuse = tile && m->sen_is_cb && m->n_mgau > 1;
         MsSenArgs sa = {m->d_mixw, m->d_logadd_ms, m->logadd_ms_size, m->logadd_ms_zero, d_senscr, b->d_msbest, n_used, m->aw};
         if (fuse) {
             fill_i32<<<(unsigned)((n + 255) / 256), 256, 0, b->stream>>>(b->d_msbest, n, 0x7fffffff);
             PSB_LAUNCH_CHECK();
         }
-#define PSB_MS_TILE(NT, TFT, PKV, FUSEV) do {                                                                              \
-            auto kern = ms_dist_tile_kernel<NT, TFT, PKV, FUSEV>;                                                         \
+#define PSB_MS_TILE(NT, FUSEV) do {                                                                                        \
+            auto kern = ms_dist_tile_kernel<NT, FUSEV>;                                                                   \
             PSB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tile_smem));            \
-            kern<<<gt, MS_TFB / TFT * 32, tile_smem, b->stream>>>(m->d_msT, m->d_msdetT, d_feats, dist, f0, n, m->n_mgau, \
-                m->n_feat, m->n_density, m->sumlen, m->d_featlen, m->d_featoff, (int)fpc, sa); } while (0)
-#define LAUNCH(NT) do { if (tile) {                                                                                       \
-            if (fuse) PSB_MS_TILE(NT, 4, true, true);                                                                      \
-            else if (tile_tft4 && tile_pk) PSB_MS_TILE(NT, 4, true, false);                                                \
-            else if (tile_tft4) PSB_MS_TILE(NT, 4, false, false);                                                          \
-            else if (tile_pk) PSB_MS_TILE(NT, 8, true, false);                                                             \
-            else PSB_MS_TILE(NT, 8, false, false); }                                                                       \
-        else if (reg_tile && m->n_density <= ND_MAX)                                                          \
-            ms_dist_reg_kernel<NT><<<g1, 128, smem, b->stream>>>(m->d_msT, m->d_msdetT, d_feats, dist, f0, n,             \
-                m->n_mgau, m->n_feat, m->n_density, m->sumlen, m->d_featlen, m->d_featoff);                             \
-        else if (packed) ms_dist2_kernel<NT><<<g1, 128, smem, b->stream>>>(m->d_msT, m->d_msdetT, d_feats, dist, f0, n,   \
-                m->n_mgau, m->n_feat, m->n_density, m->sumlen, m->d_featlen, m->d_featoff);                             \
-        else ms_dist_kernel<NT><<<g1, 128, smem, b->stream>>>(m->d_msT, m->d_msdetT, d_feats, dist, f0, n,                \
+            kern<<<gt, MS_TFB / MS_TFT * 32, tile_smem, b->stream>>>(m->d_msT, m->d_msdetT, d_feats, dist, f0, n,         \
+                m->n_mgau, m->n_feat, m->n_density, m->sumlen, m->d_featlen, m->d_featoff, (int)fpc, sa); } while (0)
+#define LAUNCH(NT) do {                                                                                                    \
+            if (fuse) PSB_MS_TILE(NT, true);                                                                               \
+            else if (tile) PSB_MS_TILE(NT, false);                                                                         \
+            else ms_dist_kernel<NT><<<g1, 128, smem, b->stream>>>(m->d_msT, m->d_msdetT, d_feats, dist, f0, n,            \
                 m->n_mgau, m->n_feat, m->n_density, m->sumlen, m->d_featlen, m->d_featoff); } while (0)
         switch (nt) {
         case 1: LAUNCH(1); break;
@@ -623,7 +413,7 @@ int psb_launch_ms_batch(psb_batch_t *b, const float *d_feats, const int32_t *utt
 #undef PSB_MS_TILE
         PSB_LAUNCH_CHECK();
         dim3 g2((m->n_sen + 255) / 256, (unsigned)n);
-        if (!(tile && fuse)) {
+        if (!fuse) {
             fill_i32<<<(unsigned)((n + 255) / 256), 256, 0, b->stream>>>(b->d_msbest, n, 0x7fffffff);
             PSB_LAUNCH_CHECK();
             ms_senone_kernel<<<g2, 256, 0, b->stream>>>(dist, m->d_mixw, m->d_sen2cb32, m->d_logadd_ms, m->logadd_ms_size,

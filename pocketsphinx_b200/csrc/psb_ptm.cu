@@ -30,7 +30,7 @@
 namespace {
 
 constexpr int TOPN = 4;               // kernels below are specialised for -topn 4 (the default)
-constexpr int TOPN_WARPS = 4;         // warps per CTA in ptm_topn_kernel
+constexpr int TOPN_WARPS = 4;         // warps per CTA of the scan kernels
 constexpr int MAX_NDW = 8;            // up to 256 codewords per codebook
 
 // FIXED_POINT build of the reference (mfcc_t = int32 Q12, SURVEY A.1.11): the same records and the
@@ -283,8 +283,10 @@ ptm_topn_kernel(const float *__restrict__ rec, const size_t *__restrict__ rec_of
     }
 }
 
-template <int FL, bool SEMI, int WARPS, int MINB>
-__global__ void __launch_bounds__(WARPS * 32, MINB)
+// The scan of ptm_topn_kernel<FL, true> with two codewords per packed distance (pair records, FADD2 / FMUL2): the
+// semi-continuous models the split path below does not take.
+template <int FL>
+__global__ void __launch_bounds__(TOPN_WARPS * 32, 7)
 ptm_topn2_kernel(const float *__restrict__ rec2, const size_t *__restrict__ rec2_off,
                  const int32_t *__restrict__ klist, const float *__restrict__ featT, GroupTabs tabs,
                  int4 *__restrict__ out, int n_groups, int nd, int n_feat, int D,
@@ -302,7 +304,7 @@ ptm_topn2_kernel(const float *__restrict__ rec2, const size_t *__restrict__ rec2
             srec[i] = src[i];
     }
     __syncthreads();
-    const int g = blockIdx.y * WARPS + warp;
+    const int g = blockIdx.y * TOPN_WARPS + warp;
     if (g >= n_groups) return;
     const int len = tabs.lane_len[g * 32 + lane];
     const long long off = tabs.lane_off[g * 32 + lane];
@@ -369,14 +371,12 @@ ptm_topn2_kernel(const float *__restrict__ rec2, const size_t *__restrict__ rec2
 #pragma unroll
                 for (int pp = 0; pp < 4; ++pp) {
                     float2 dpen2;
-                    const float2 d2 = gau_dist2<FL, SEMI>(rq + pp * RECQ2, xx, &dpen2);
+                    const float2 d2 = gau_dist2<FL, true>(rq + pp * RECQ2, xx, &dpen2);
 #pragma unroll
                     for (int h = 0; h < 2; ++h) {
                         const int cc = 2 * pp + h;
                         const float d = h ? d2.y : d2.x;
-                        bool hit;
-                        if (SEMI) hit = (h ? dpen2.y : dpen2.x) >= thresh && f2i_clamped(d) >= sc[TOPN - 1];
-                        else hit = d >= thresh;
+                        const bool hit = (h ? dpen2.y : dpen2.x) >= thresh && f2i_clamped(d) >= sc[TOPN - 1];
                         if (hit && !(m8 & (1u << cc))) {
                             const int c = ch * 8 + cc;
                             const int s = f2i_clamped(d);
@@ -403,219 +403,20 @@ ptm_topn2_kernel(const float *__restrict__ rec2, const size_t *__restrict__ rec2
             }
         }
 
-        // ---- emit the record (same format as ptm_topn_kernel) ----
+        // ---- emit the record (same format as ptm_topn_kernel<FL, true>) ----
         const int top = sc[0] >> PSB_SENSCR_SHIFT;
         unsigned cwb = 0, eb = 0;
         int n_in_beam = TOPN;
 #pragma unroll
         for (int j = 0; j < TOPN; ++j) {
             int e = top - (sc[j] >> PSB_SENSCR_SHIFT);
-            if (SEMI) {
-                e = e > PSB_MAX_NEG_ASCR ? PSB_MAX_NEG_ASCR : e;
-                const int beam = topn_beam[f];
-                if (beam && e > beam && n_in_beam == TOPN) n_in_beam = j;
-            }
-            else
-                e = e > 255 ? 255 : e;
+            e = e > PSB_MAX_NEG_ASCR ? PSB_MAX_NEG_ASCR : e;
+            const int beam = topn_beam[f];
+            if (beam && e > beam && n_in_beam == TOPN) n_in_beam = j;
             cwb |= (unsigned)cw[j] << (8 * j);
             eb |= (unsigned)e << (8 * j);
         }
-        out[(off + t) * K + k] = make_int4(SEMI ? n_in_beam : top, (int)cwb, (int)eb, 0);
-    }
-}
-
-// ---------------------------------------------------------------------------------------
-// Two utterances per lane ("U2").  ncu on the kernels above shows the warp-uniform LDS.128
-// stream of Gaussian records at ~65 % of the shared-memory pipe with `short scoreboard` the top
-// stall: a broadcast load delivers 8 bytes per wavefront however many lanes listen.  Here every
-// record load feeds TWO utterances per lane: the pair (x_u0, x_u1) goes through one
-// FADD2 / FMUL2 / FMUL2 with the model value as a broadcast scalar operand (so the scalar records
-// are used as they are: t = x + (-mu), t*t, (t*t)*v, then d_u -= t_u with scalar FADDs, which
-// ptxas never contracts).  Shared-memory traffic per (utterance, codeword) halves and each warp
-// carries two independent dependency chains.
-struct U2State {
-    unsigned cwp;           // four listed codewords, byte j = cw_j
-    int sc[TOPN];
-    unsigned seedpack, seedbit;
-    float thresh;
-};
-
-__device__ __forceinline__ void u2_insert(U2State &st, int c, int s, int ch, unsigned &m8)
-{
-    const int ev = (int)(st.cwp >> 24);
-    int p = 0;
-#pragma unroll
-    for (int j = 0; j < TOPN - 1; ++j) p += (s >= st.sc[j]) ? 0 : 1;       // insertion_sort_cb (ptm_mgau.c:140-149)
-#pragma unroll
-    for (int j = TOPN - 2; j >= 0; --j)
-        if (j >= p) st.sc[j + 1] = st.sc[j];
-#pragma unroll
-    for (int j = 0; j < TOPN; ++j)
-        if (j == p) st.sc[j] = s;
-    const unsigned lowmask = (1u << (8 * p)) - 1u;                          // p <= 3
-    st.cwp = (st.cwp & lowmask) | ((unsigned)c << (8 * p)) | ((st.cwp << 8) & ~((lowmask << 8) | 0xffu));
-    // an evicted seed becomes scannable again (it may lie ahead of the scan)
-    const unsigned t2 = st.seedpack ^ ((unsigned)ev * 0x01010101u);
-    const unsigned nz2 = (((t2 & 0x7f7f7f7fu) + 0x7f7f7f7fu) | t2) & 0x80808080u;
-    st.seedbit &= (nz2 >> 7) * 0xffu;
-    if ((ev >> 3) == ch) m8 &= ~(1u << (ev & 7));
-    st.thresh = (float)st.sc[TOPN - 1];
-}
-
-template <int FL, bool SEMI>
-__global__ void __launch_bounds__(128, 5)
-ptm_topn_u2_kernel(const float *__restrict__ rec, const size_t *__restrict__ rec_off,
-                   const int32_t *__restrict__ klist, const float *__restrict__ featT, GroupTabs tabs,
-                   int4 *__restrict__ out, int n_groups, int nd, int n_feat, int D,
-                   const int32_t *__restrict__ featoff, int K, int ds_ratio, const int32_t *__restrict__ topn_beam)
-{
-    constexpr int RECF = (1 + 2 * FL + 3) / 4 * 4;
-    constexpr int RECQ = RECF / 4;
-    extern __shared__ float4 srec[];          // [nd][RECQ] scalar records {det, mu0, v0, ...}
-    const int k = klist[blockIdx.x];
-    const int f = k % n_feat;
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    {
-        const float4 *src = reinterpret_cast<const float4 *>(rec + rec_off[k]);
-        for (int i = threadIdx.x; i < nd * RECQ; i += blockDim.x)
-            srec[i] = src[i];
-    }
-    __syncthreads();
-    // this warp owns utterance groups g0 = 2w and g1 = 2w + 1 (the second may not exist)
-    const int w = blockIdx.y * (blockDim.x >> 5) + warp;
-    const int g0 = 2 * w, g1 = 2 * w + 1;
-    if (g0 >= n_groups) return;
-    const bool has1 = g1 < n_groups;
-    const int len0 = tabs.lane_len[g0 * 32 + lane], len1 = has1 ? tabs.lane_len[g1 * 32 + lane] : 0;
-    const long long off0 = tabs.lane_off[g0 * 32 + lane], off1 = has1 ? tabs.lane_off[g1 * 32 + lane] : 0;
-    const int maxT = max(tabs.grp_maxT[g0], has1 ? tabs.grp_maxT[g1] : 0);
-    const int maxT1 = has1 ? tabs.grp_maxT[g1] : 0, maxT0 = tabs.grp_maxT[g0];
-    const float *xT0 = featT + tabs.grp_base[g0] + (long long)featoff[f] * 32 + lane;
-    const float *xT1 = has1 ? featT + tabs.grp_base[g1] + (long long)featoff[f] * 32 + lane : xT0;
-
-    U2State st[2];
-#pragma unroll
-    for (int u = 0; u < 2; ++u) {
-        st[u].cwp = 0x03020100u;                                   // codewords 0..3 (ptm_mgau.c:791-792)
-#pragma unroll
-        for (int i = 0; i < TOPN; ++i) st[u].sc[i] = INT_MIN;
-        st[u].seedpack = st[u].seedbit = 0u;
-        st[u].thresh = 0.f;
-    }
-
-    for (int t = 0; t < maxT; ++t) {
-        float2 xx[FL];
-        {
-            const float *p0 = xT0 + (long long)t * D * 32, *p1 = xT1 + (long long)t * D * 32;
-            const bool in0 = t < maxT0, in1 = t < maxT1;
-#pragma unroll
-            for (int j = 0; j < FL; ++j) xx[j] = make_float2(in0 ? p0[j * 32] : 0.f, in1 ? p1[j * 32] : 0.f);
-        }
-        const bool act0 = t < len0, act1 = t < len1;
-        if (!act0 && !act1) continue;
-
-        // ---- eval_topn per utterance (scalar distances through per-lane record addresses) ----
-#pragma unroll
-        for (int u = 0; u < 2; ++u) {
-            float x[FL];
-#pragma unroll
-            for (int j = 0; j < FL; ++j) x[j] = u ? xx[j].y : xx[j].x;
-            int ncw[TOPN], nsc[TOPN];
-            unsigned sp = 0u, sb = 0u;
-#pragma unroll
-            for (int i = 0; i < TOPN; ++i) {
-                const int c = (st[u].cwp >> (8 * i)) & 0xff;
-                const int s = f2i_clamped(gau_dist<FL>(srec + c * RECQ, x));
-                sp |= (unsigned)c << (8 * i);
-                sb |= (1u << (c & 7)) << (8 * i);
-                int p = 0;
-#pragma unroll
-                for (int j = 0; j < i; ++j) p += (s > nsc[j]) ? 0 : 1;
-#pragma unroll
-                for (int j = TOPN - 2; j >= 0; --j)
-                    if (j < i && j >= p) { nsc[j + 1] = nsc[j]; ncw[j + 1] = ncw[j]; }
-#pragma unroll
-                for (int j = 0; j < TOPN; ++j)
-                    if (j == p) { nsc[j] = s; ncw[j] = c; }
-            }
-            unsigned cp = 0u;
-#pragma unroll
-            for (int i = 0; i < TOPN; ++i) { st[u].sc[i] = nsc[i]; cp |= (unsigned)ncw[i] << (8 * i); }
-            st[u].cwp = cp;
-            st[u].seedpack = sp;
-            st[u].seedbit = sb;
-            st[u].thresh = (float)nsc[TOPN - 1];
-        }
-
-        // ---- eval_cb: one record stream, two utterances ----
-        if (t % ds_ratio == 0) {
-            const unsigned sch0 = (st[0].seedpack >> 3) & 0x1f1f1f1fu, sch1 = (st[1].seedpack >> 3) & 0x1f1f1f1fu;
-            for (int ch = 0; ch < nd / 8; ++ch) {
-                const float4 *rq = srec + (size_t)ch * 8 * RECQ;
-                unsigned m8[2];
-#pragma unroll
-                for (int u = 0; u < 2; ++u) {
-                    const unsigned tt = (u ? sch1 : sch0) ^ ((unsigned)ch * 0x01010101u);
-                    const unsigned nz = (((tt & 0x7f7f7f7fu) + 0x7f7f7f7fu) | tt) & 0x80808080u;
-                    const unsigned b = st[u].seedbit & (((nz ^ 0x80808080u) >> 7) * 0xffu);
-                    m8[u] = (b | (b >> 8) | (b >> 16) | (b >> 24)) & 0xffu;
-                }
-                if (!act0) m8[0] = 0xffu;          // a finished utterance never inserts
-                if (!act1) m8[1] = 0xffu;
-#pragma unroll 2
-                for (int cc = 0; cc < 8; ++cc) {
-                    const float4 *r = rq + cc * RECQ;
-                    float rr[RECF];
-#pragma unroll
-                    for (int q = 0; q < RECQ; ++q) {
-                        const float4 v = r[q];
-                        rr[4 * q] = v.x; rr[4 * q + 1] = v.y; rr[4 * q + 2] = v.z; rr[4 * q + 3] = v.w;
-                    }
-                    float d0 = rr[0], d1 = rr[0], p0 = rr[0], p1 = rr[0];
-#pragma unroll
-                    for (int j = 0; j < FL; ++j) {
-                        float2 tt = __fadd2_rn(xx[j], make_float2(-rr[1 + 2 * j], -rr[1 + 2 * j]));
-                        tt = __fmul2_rn(tt, tt);
-                        tt = __fmul2_rn(tt, make_float2(rr[2 + 2 * j], rr[2 + 2 * j]));
-                        if (SEMI && j == FL - 1) { p0 = d0; p1 = d1; }
-                        d0 = __fsub_rn(d0, tt.x);
-                        d1 = __fsub_rn(d1, tt.y);
-                    }
-                    const int c = ch * 8 + cc;
-#pragma unroll
-                    for (int u = 0; u < 2; ++u) {
-                        const float d = u ? d1 : d0;
-                        bool hit;
-                        if (SEMI) hit = (u ? p1 : p0) >= st[u].thresh && f2i_clamped(d) >= st[u].sc[TOPN - 1];
-                        else hit = d >= st[u].thresh;
-                        if (hit && !((m8[u] >> cc) & 1u))
-                            u2_insert(st[u], c, f2i_clamped(d), ch, m8[u]);
-                    }
-                }
-            }
-        }
-
-        // ---- emit the records ----
-#pragma unroll
-        for (int u = 0; u < 2; ++u) {
-            if (u ? !act1 : !act0) continue;
-            const int top = st[u].sc[0] >> PSB_SENSCR_SHIFT;
-            unsigned eb = 0;
-            int n_in_beam = TOPN;
-#pragma unroll
-            for (int j = 0; j < TOPN; ++j) {
-                int e = top - (st[u].sc[j] >> PSB_SENSCR_SHIFT);
-                if (SEMI) {
-                    e = e > PSB_MAX_NEG_ASCR ? PSB_MAX_NEG_ASCR : e;
-                    const int beam = topn_beam[f];
-                    if (beam && e > beam && n_in_beam == TOPN) n_in_beam = j;
-                }
-                else
-                    e = e > 255 ? 255 : e;
-                eb |= (unsigned)e << (8 * j);
-            }
-            out[((u ? off1 : off0) + t) * K + k] = make_int4(SEMI ? n_in_beam : top, (int)st[u].cwp, (int)eb, 0);
-        }
+        out[(off + t) * K + k] = make_int4(n_in_beam, (int)cwb, (int)eb, 0);
     }
 }
 
@@ -624,10 +425,8 @@ ptm_topn_u2_kernel(const float *__restrict__ rec, const size_t *__restrict__ rec
 // are NOT distance arithmetic -- the insertion path runs for a warp whenever ANY of its 32
 // utterances accepts the current codeword (~80 of 256 codewords per frame), each time with one
 // or two lanes live -- and the warp-uniform LDS.128 record stream sits at 64 % of the
-// shared-memory data pipe (a broadcast delivers 8 bytes per wavefront).  Two changes:
-//  * NU utterances per lane share every record load: the pair record {A,B} is used as is, each
-//    utterance keeps its own duplicated feature registers (x,x), so there is no repacking and
-//    LDS traffic per (utterance, codeword) drops by NU.
+// shared-memory data pipe (a broadcast delivers 8 bytes per wavefront).  The pair record {A,B}
+// is used as is with duplicated feature registers (x,x), so there is no repacking, and:
 //  * The scan only FILTERS: a codeword whose distance passes `d >= thresh` against a stale
 //    (= lower or equal, the worst score only rises during a scan) threshold is pushed on a small
 //    per-utterance queue in shared memory (distance) and a register (codeword byte).  All lanes
@@ -695,8 +494,8 @@ __device__ __forceinline__ void q_drain(QState &st, unsigned q, bool active)
     if (active) st.thresh = (float)st.sc[TOPN - 1];
 }
 
-template <int FL, int NU, int WARPS, int MINB>
-__global__ void __launch_bounds__(WARPS * 32, MINB)
+template <int FL>
+__global__ void __launch_bounds__(TOPN_WARPS * 32, 7)
 ptm_topnq_kernel(const float *__restrict__ rec2, const size_t *__restrict__ rec2_off,
                  const int32_t *__restrict__ klist, const float *__restrict__ featT, GroupTabs tabs,
                  int4 *__restrict__ out, int n_groups, int nd, int n_feat, int D,
@@ -704,12 +503,11 @@ ptm_topnq_kernel(const float *__restrict__ rec2, const size_t *__restrict__ rec2
 {
     constexpr int RECF2 = (2 + 4 * FL + 3) / 4 * 4;
     constexpr int RECQ2 = RECF2 / 4;
-    constexpr int NT = WARPS * 32;
+    constexpr int NT = TOPN_WARPS * 32;
     constexpr unsigned FULL = 0xffffffffu;
-    extern __shared__ float4 srec[];          // [nd/2][RECQ2] pair records, then float q[NU][QCAP][NT]
+    extern __shared__ float4 srec[];          // [nd/2][RECQ2] pair records, then float q[QCAP][NT]
     const unsigned qbase = (unsigned)__cvta_generic_to_shared(
         reinterpret_cast<float *>(srec + (size_t)(nd >> 1) * RECQ2) + threadIdx.x);
-    constexpr unsigned QU = QCAP * NT * 4;      // bytes between the queues of two utterances of a lane
     const int k = klist[blockIdx.x];
     const int f = k % n_feat;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -719,60 +517,41 @@ ptm_topnq_kernel(const float *__restrict__ rec2, const size_t *__restrict__ rec2
             srec[i] = src[i];
     }
     __syncthreads();
-    // this warp owns utterance groups NU*w .. NU*w + NU-1 (the trailing ones may not exist)
-    const int w = blockIdx.y * WARPS + warp;
-    if (NU * w >= n_groups) return;
-    int len[NU], gmaxT[NU];
-    long long off[NU];
-    const float *xT[NU];
-    int maxT = 0;
-#pragma unroll
-    for (int u = 0; u < NU; ++u) {
-        const int g = NU * w + u;
-        const bool has = g < n_groups;
-        len[u] = has ? tabs.lane_len[g * 32 + lane] : 0;
-        off[u] = has ? tabs.lane_off[g * 32 + lane] : 0;
-        gmaxT[u] = has ? tabs.grp_maxT[g] : 0;
-        xT[u] = featT + (has ? tabs.grp_base[g] : 0) + (long long)featoff[f] * 32 + lane;
-        maxT = max(maxT, gmaxT[u]);
-    }
+    const int g = blockIdx.y * TOPN_WARPS + warp;
+    if (g >= n_groups) return;
+    const int len = tabs.lane_len[g * 32 + lane];
+    const long long off = tabs.lane_off[g * 32 + lane];
+    const int maxT = max(0, tabs.grp_maxT[g]);
+    const float *xT = featT + tabs.grp_base[g] + (long long)featoff[f] * 32 + lane;
 
-    QState st[NU];
+    QState st;
+    st.cwp = 0x03020100u;                                          // codewords 0..3 (ptm_mgau.c:791-792)
 #pragma unroll
-    for (int u = 0; u < NU; ++u) {
-        st[u].cwp = 0x03020100u;                                   // codewords 0..3 (ptm_mgau.c:791-792)
-#pragma unroll
-        for (int i = 0; i < TOPN; ++i) st[u].sc[i] = INT_MIN;
-        st[u].thresh = 0.f;
-        st[u].qc = 0u;
-        st[u].qw = qbase + u * QU;
-    }
+    for (int i = 0; i < TOPN; ++i) st.sc[i] = INT_MIN;
+    st.thresh = 0.f;
+    st.qc = 0u;
+    st.qw = qbase;
 
     for (int t = 0; t < maxT; ++t) {
-        float2 xx[NU][FL];
-        bool act[NU], any = false;
-#pragma unroll
-        for (int u = 0; u < NU; ++u) {
-            const float *p = xT[u] + (long long)t * D * 32;
-            const bool in = t < gmaxT[u];
+        float2 xx[FL];
+        {
+            const float *p = xT + (long long)t * D * 32;
 #pragma unroll
             for (int j = 0; j < FL; ++j) {
-                const float v = in ? p[j * 32] : 0.f;
-                xx[u][j] = make_float2(v, v);
+                const float v = p[j * 32];
+                xx[j] = make_float2(v, v);
             }
-            act[u] = t < len[u];
-            any |= act[u];
         }
-        if (!__any_sync(FULL, any)) continue;                       // warp-uniform: the votes below need all lanes
+        const bool act = t < len;
+        if (!__any_sync(FULL, act)) continue;                       // warp-uniform: the votes below need all lanes
 
-        // ---- eval_topn per utterance: re-score the listed codewords (ptm_mgau.c:88-135) ----
-#pragma unroll
-        for (int u = 0; u < NU; ++u) {
+        // ---- eval_topn: re-score the listed codewords (ptm_mgau.c:88-135) ----
+        {
             int ncw[TOPN], nsc[TOPN];
 #pragma unroll
             for (int i = 0; i < TOPN; ++i) {
-                const int c = (st[u].cwp >> (8 * i)) & 0xff;
-                const float2 d2 = gau_dist2<FL>(srec + (c >> 1) * RECQ2, xx[u]);
+                const int c = (st.cwp >> (8 * i)) & 0xff;
+                const float2 d2 = gau_dist2<FL>(srec + (c >> 1) * RECQ2, xx);
                 const int s = f2i_clamped((c & 1) ? d2.y : d2.x);
                 int p = 0;
 #pragma unroll
@@ -786,12 +565,12 @@ ptm_topnq_kernel(const float *__restrict__ rec2, const size_t *__restrict__ rec2
             }
             unsigned cp = 0u;
 #pragma unroll
-            for (int i = 0; i < TOPN; ++i) { st[u].sc[i] = nsc[i]; cp |= (unsigned)ncw[i] << (8 * i); }
-            st[u].cwp = cp;
-            st[u].thresh = act[u] ? (float)nsc[TOPN - 1] : __int_as_float(0x7f800000);
+            for (int i = 0; i < TOPN; ++i) { st.sc[i] = nsc[i]; cp |= (unsigned)ncw[i] << (8 * i); }
+            st.cwp = cp;
+            st.thresh = act ? (float)nsc[TOPN - 1] : __int_as_float(0x7f800000);
         }
 
-        // ---- eval_cb: filter in codeword order, one record stream for NU utterances ----
+        // ---- eval_cb: filter in codeword order ----
         if (t % ds_ratio == 0) {
 #pragma unroll 2
             for (int pp = 0; pp < (nd >> 1); ++pp) {
@@ -803,63 +582,43 @@ ptm_topnq_kernel(const float *__restrict__ rec2, const size_t *__restrict__ rec2
                     rr[2 * q] = make_float2(v.x, v.y);
                     rr[2 * q + 1] = make_float2(v.z, v.w);
                 }
-                float2 d[NU];
-#pragma unroll
-                for (int u = 0; u < NU; ++u) d[u] = rr[0];
+                float2 d = rr[0];
 #pragma unroll
                 for (int j = 0; j < FL; ++j) {
-#pragma unroll
-                    for (int u = 0; u < NU; ++u) {
-                        float2 tt = __fadd2_rn(xx[u][j], rr[1 + 2 * j]);
-                        tt = __fmul2_rn(tt, tt);
-                        tt = __fmul2_rn(tt, rr[2 + 2 * j]);
-                        d[u].x = __fadd_rn(d[u].x, tt.x);             // scalar on purpose: see gau_dist2
-                        d[u].y = __fadd_rn(d[u].y, tt.y);
-                    }
+                    float2 tt = __fadd2_rn(xx[j], rr[1 + 2 * j]);
+                    tt = __fmul2_rn(tt, tt);
+                    tt = __fmul2_rn(tt, rr[2 + 2 * j]);
+                    d.x = __fadd_rn(d.x, tt.x);                        // scalar on purpose: see gau_dist2
+                    d.y = __fadd_rn(d.y, tt.y);
                 }
-                bool full = false;
-#pragma unroll
-                for (int u = 0; u < NU; ++u) {
-                    if (d[u].x >= st[u].thresh) {
-                        sts_f32(st[u].qw, d[u].x);
-                        st[u].qc = __byte_perm(st[u].qc, (unsigned)(2 * pp), 0x2104);
-                        st[u].qw += NT * 4;
-                    }
-                    if (d[u].y >= st[u].thresh) {
-                        sts_f32(st[u].qw, d[u].y);
-                        st[u].qc = __byte_perm(st[u].qc, (unsigned)(2 * pp + 1), 0x2104);
-                        st[u].qw += NT * 4;
-                    }
-                    full |= st[u].qw > qbase + u * QU + (QCAP - 2) * NT * 4;
+                if (d.x >= st.thresh) {
+                    sts_f32(st.qw, d.x);
+                    st.qc = __byte_perm(st.qc, (unsigned)(2 * pp), 0x2104);
+                    st.qw += NT * 4;
                 }
-                if (__any_sync(FULL, full)) {
-#pragma unroll
-                    for (int u = 0; u < NU; ++u) q_drain<NT>(st[u], qbase + u * QU, act[u]);
+                if (d.y >= st.thresh) {
+                    sts_f32(st.qw, d.y);
+                    st.qc = __byte_perm(st.qc, (unsigned)(2 * pp + 1), 0x2104);
+                    st.qw += NT * 4;
                 }
+                if (__any_sync(FULL, st.qw > qbase + (QCAP - 2) * NT * 4))
+                    q_drain<NT>(st, qbase, act);
             }
-            bool pend = false;
-#pragma unroll
-            for (int u = 0; u < NU; ++u) pend |= st[u].qw != qbase + u * QU;
-            if (__any_sync(FULL, pend)) {
-#pragma unroll
-                for (int u = 0; u < NU; ++u) q_drain<NT>(st[u], qbase + u * QU, act[u]);
-            }
+            if (__any_sync(FULL, st.qw != qbase))
+                q_drain<NT>(st, qbase, act);
         }
 
-        // ---- emit the records (same format as ptm_topn_kernel) ----
+        // ---- emit the record (same format as ptm_topn_kernel) ----
+        if (!act) continue;
+        const int top = st.sc[0] >> PSB_SENSCR_SHIFT;
+        unsigned eb = 0;
 #pragma unroll
-        for (int u = 0; u < NU; ++u) {
-            if (!act[u]) continue;
-            const int top = st[u].sc[0] >> PSB_SENSCR_SHIFT;
-            unsigned eb = 0;
-#pragma unroll
-            for (int j = 0; j < TOPN; ++j) {
-                int e = top - (st[u].sc[j] >> PSB_SENSCR_SHIFT);
-                e = e > 255 ? 255 : e;
-                eb |= (unsigned)e << (8 * j);
-            }
-            out[(off[u] + t) * K + k] = make_int4(top, (int)st[u].cwp, (int)eb, 0);
+        for (int j = 0; j < TOPN; ++j) {
+            int e = top - (st.sc[j] >> PSB_SENSCR_SHIFT);
+            e = e > 255 ? 255 : e;
+            eb |= (unsigned)e << (8 * j);
         }
+        out[(off + t) * K + k] = make_int4(top, (int)st.cwp, (int)eb, 0);
     }
 }
 
@@ -1167,10 +926,6 @@ semi_senone_kernel(const int4 *__restrict__ topn, const uint8_t *__restrict__ mi
 // owns senones 4q..4q+3 fetches each weight row with ONE aligned 32-bit load (four senones'
 // bytes) and reads the codebook's offsets/scores once; quads that straddle a codebook boundary
 // (a few per cent) take the per-senone path.
-// TAB2: the add table is zero from entry 31 on (every logbase-1.0001 >> 10 table is), so the two look-ups of a packed
-// log-add -- tab[d_lo] and tab[d_hi] -- become ONE 32-bit read of a 32 x 32 table of ready-made halfword pairs indexed
-// by the two differences clamped to 31: half the shared-memory instructions of the loop (its limit: LSU data pipe 84 %).
-template <bool TAB2>
 __global__ void __launch_bounds__(512)
 ptm_senone4_kernel(const int4 *__restrict__ topn, const uint8_t *__restrict__ mixw,
                    const uint16_t *__restrict__ sen2cb, const int16_t *__restrict__ quadcb,
@@ -1187,13 +942,10 @@ ptm_senone4_kernel(const int4 *__restrict__ topn, const uint8_t *__restrict__ mi
     int *red = norm + 8;                                            // [32]
     uint8_t *tab = reinterpret_cast<uint8_t *>(red + 32);           // [PSB_LOGADD8_N]
     int16_t *asc = reinterpret_cast<int16_t *>(tab + PSB_LOGADD8_N + 16);     // [n_sen rounded up to 4]
-    unsigned *tab2 = reinterpret_cast<unsigned *>(asc + ((n_sen + 7) & ~7));  // [32 * 32] (TAB2 only)
     const long long frame = blockIdx.x;
     const int tid = threadIdx.x;
 
     for (int i = tid; i < PSB_LOGADD8_N; i += blockDim.x) tab[i] = logadd_tab[i];
-    if (TAB2)
-        for (int i = tid; i < 1024; i += blockDim.x) tab2[i] = (unsigned)logadd_tab[i & 31] | ((unsigned)logadd_tab[i >> 5] << 16);
     if (tid < n_feat) norm[tid] = PSB_WORST_SCORE;
     __syncthreads();
     int4 r = make_int4(0, 0, 0, 0);
@@ -1245,13 +997,7 @@ ptm_senone4_kernel(const int4 *__restrict__ topn, const uint8_t *__restrict__ mi
                 const unsigned mn = __viaddmin_u16x2(y, nvj, x);                                \
                 const unsigned mx = __viaddmax_u16x2(y, nvj, x);                                \
                 const unsigned d = mx - mn;                                                     \
-                unsigned t;                                                                     \
-                if (TAB2) {                                                                     \
-                    const unsigned dc = __vminu2(d, 0x001f001fu);                               \
-                    t = tab2[(dc & 0x1fu) | (dc >> 11)];                                        \
-                }                                                                               \
-                else                                                                            \
-                    t = (unsigned)tab[d & 0xffffu] | ((unsigned)tab[d >> 16] << 16);            \
+                const unsigned t = (unsigned)tab[d & 0xffffu] | ((unsigned)tab[d >> 16] << 16); \
                 x = mn - t;                                                                     \
             }
             PSB_LADD2(x01, w1, 0x4140, nv.y) PSB_LADD2(x23, w1, 0x4342, nv.y)
@@ -1298,95 +1044,61 @@ ptm_senone4_kernel(const int4 *__restrict__ topn, const uint8_t *__restrict__ mi
         dst[s] = (int16_t)(asc[s] - best);                       // ptm_mgau.c:398-400
 }
 
-template <int FL, bool SEMI, int WARPS, int MINB>
+template <int FL>
 int launch_topn2(psb_batch_t *b, const int32_t *d_klist, int n_k, const GroupTabs &tabs, int n_groups,
                  const int32_t *d_featoff)
 {
     psb_model_t *m = b->m;
     constexpr int RECF2 = (2 + 4 * FL + 3) / 4 * 4;
     size_t smem = (size_t)(m->n_density / 2) * RECF2 * sizeof(float);
-    auto kern = ptm_topn2_kernel<FL, SEMI, WARPS, MINB>;
+    auto kern = ptm_topn2_kernel<FL>;
     PSB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    dim3 grid(n_k, (n_groups + WARPS - 1) / WARPS);
-    kern<<<grid, WARPS * 32, smem, b->stream>>>(m->d_rec2, m->d_rec2_off, d_klist, b->d_featT, tabs, b->d_topn, n_groups,
-                                               m->n_density, m->n_feat, m->sumlen, d_featoff, m->K, m->ds_ratio,
-                                               m->d_topn_beam);
+    dim3 grid(n_k, (n_groups + TOPN_WARPS - 1) / TOPN_WARPS);
+    kern<<<grid, TOPN_WARPS * 32, smem, b->stream>>>(m->d_rec2, m->d_rec2_off, d_klist, b->d_featT, tabs, b->d_topn, n_groups,
+                                                    m->n_density, m->n_feat, m->sumlen, d_featoff, m->K, m->ds_ratio,
+                                                    m->d_topn_beam);
     PSB_LAUNCH_CHECK();
     return PSB_OK;
 }
 
-template <int FL, int NU, int WARPS, int MINB>
+template <int FL>
 int launch_topnq(psb_batch_t *b, const int32_t *d_klist, int n_k, const GroupTabs &tabs, int n_groups,
                  const int32_t *d_featoff)
 {
     psb_model_t *m = b->m;
     constexpr int RECF2 = (2 + 4 * FL + 3) / 4 * 4;
-    const size_t smem = (size_t)(m->n_density / 2) * RECF2 * sizeof(float)
-                        + (size_t)NU * QCAP * WARPS * 32 * sizeof(float);
-    auto kern = ptm_topnq_kernel<FL, NU, WARPS, MINB>;
+    const size_t smem = (size_t)(m->n_density / 2) * RECF2 * sizeof(float) + (size_t)QCAP * TOPN_WARPS * 32 * sizeof(float);
+    auto kern = ptm_topnq_kernel<FL>;
     PSB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const int n_w = (n_groups + NU - 1) / NU;
-    dim3 grid(n_k, (n_w + WARPS - 1) / WARPS);
-    kern<<<grid, WARPS * 32, smem, b->stream>>>(m->d_rec2, m->d_rec2_off, d_klist, b->d_featT, tabs, b->d_topn, n_groups,
-                                               m->n_density, m->n_feat, m->sumlen, d_featoff, m->K, m->ds_ratio);
+    dim3 grid(n_k, (n_groups + TOPN_WARPS - 1) / TOPN_WARPS);
+    kern<<<grid, TOPN_WARPS * 32, smem, b->stream>>>(m->d_rec2, m->d_rec2_off, d_klist, b->d_featT, tabs, b->d_topn, n_groups,
+                                                    m->n_density, m->n_feat, m->sumlen, d_featoff, m->K, m->ds_ratio);
     PSB_LAUNCH_CHECK();
     return PSB_OK;
 }
 
+// The scan for the streams of length FL: the scalar kernel for fixed point (integer distances) and for streams longer
+// than 16 dimensions (the packed kernels' register budget), else the packed kernels -- ptm_topnq_kernel for PTM,
+// ptm_topn2_kernel for semi-continuous models.
 template <int FL, bool SEMI>
 int launch_topn(psb_batch_t *b, const int32_t *d_klist, int n_k, const GroupTabs &tabs, int n_groups,
                 const int32_t *d_featoff)
 {
     psb_model_t *m = b->m;
-    if (m->fixed_point) {
-        // FIXED_POINT arithmetic: the scalar kernel with integer distances (one variant)
-        size_t smem = (size_t)m->n_density * rec_floats(FL) * sizeof(float);
-        auto kern = ptm_topn_kernel<FL, SEMI, true>;
-        PSB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        const int warps = (long long)n_k * ((n_groups + TOPN_WARPS - 1) / TOPN_WARPS) >= 4 * 148 ? TOPN_WARPS : 1;
-        dim3 grid(n_k, (n_groups + warps - 1) / warps);
-        kern<<<grid, warps * 32, smem, b->stream>>>(m->d_rec, m->d_rec_off, d_klist, b->d_featT, tabs, b->d_topn, n_groups,
-                                                   m->n_density, m->n_feat, m->sumlen, d_featoff, m->K, m->ds_ratio,
-                                                   m->d_topn_beam);
-        PSB_LAUNCH_CHECK();
-        return PSB_OK;
-    }
-    if (!SEMI && FL <= 16 && m->d_rec2 && b->topn_variant >= 4) {
-        // deferred-insertion kernels: 4 = two utterances per lane, 5 = one
-        constexpr int FLQ = FL <= 16 ? FL : 1;
-        if (b->topn_variant == 4) return launch_topnq<FLQ, 2, 2, 7>(b, d_klist, n_k, tabs, n_groups, d_featoff);
-        return launch_topnq<FLQ, 1, 4, 7>(b, d_klist, n_k, tabs, n_groups, d_featoff);
-    }
-    if (FL <= 16 && b->topn_variant == 3) {
-        // two utterances per lane: 64 utterances per warp, 4 warps per CTA
-        constexpr int FLU = FL <= 16 ? FL : 1;
-        size_t smem = (size_t)m->n_density * rec_floats(FLU) * sizeof(float);
-        auto kern = ptm_topn_u2_kernel<FLU, SEMI>;
-        PSB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        const int n_w = (n_groups + 1) / 2;
-        const int warps = (long long)n_k * ((n_w + 3) / 4) >= 2 * 148 ? 4 : 1;
-        dim3 grid(n_k, (n_w + warps - 1) / warps);
-        kern<<<grid, warps * 32, smem, b->stream>>>(m->d_rec, m->d_rec_off, d_klist, b->d_featT, tabs, b->d_topn, n_groups,
-                                                   m->n_density, m->n_feat, m->sumlen, d_featoff, m->K, m->ds_ratio,
-                                                   m->d_topn_beam);
-        PSB_LAUNCH_CHECK();
-        return PSB_OK;
-    }
-    if (FL <= 16 && m->d_rec2 && b->topn_variant != 0) {
-        // packed-FP32 kernels (FL <= 16 keeps the register budget): variant 1 = 2 warps/CTA with a
-        // large register budget (two balanced waves), variant 2 = 4 warps/CTA at 72 registers
-        if (b->topn_variant != 1) return launch_topn2<FL <= 16 ? FL : 1, SEMI, 4, 7>(b, d_klist, n_k, tabs, n_groups, d_featoff);
-        return launch_topn2<FL <= 16 ? FL : 1, SEMI, 2, 7>(b, d_klist, n_k, tabs, n_groups, d_featoff);
-    }
+    constexpr int FLP = FL <= 16 ? FL : 1;
+    if (FL <= 16 && !m->fixed_point)
+        return SEMI ? launch_topn2<FLP>(b, d_klist, n_k, tabs, n_groups, d_featoff)
+                    : launch_topnq<FLP>(b, d_klist, n_k, tabs, n_groups, d_featoff);
     size_t smem = (size_t)m->n_density * rec_floats(FL) * sizeof(float);
-    PSB_CUDA(cudaFuncSetAttribute(ptm_topn_kernel<FL, SEMI>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    auto kern = m->fixed_point ? ptm_topn_kernel<FL, SEMI, true> : ptm_topn_kernel<FL, SEMI, false>;
+    PSB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     // few (pair, group) items (semi-continuous models, small batches): one warp per CTA spreads
     // them over more SMs; otherwise 4 warps share one staged codebook
     const int warps = (long long)n_k * ((n_groups + TOPN_WARPS - 1) / TOPN_WARPS) >= 4 * 148 ? TOPN_WARPS : 1;
     dim3 grid(n_k, (n_groups + warps - 1) / warps);
-    ptm_topn_kernel<FL, SEMI><<<grid, warps * 32, smem, b->stream>>>(
-        m->d_rec, m->d_rec_off, d_klist, b->d_featT, tabs, b->d_topn, n_groups, m->n_density,
-        m->n_feat, m->sumlen, d_featoff, m->K, m->ds_ratio, m->d_topn_beam);
+    kern<<<grid, warps * 32, smem, b->stream>>>(m->d_rec, m->d_rec_off, d_klist, b->d_featT, tabs, b->d_topn, n_groups,
+                                               m->n_density, m->n_feat, m->sumlen, d_featoff, m->K, m->ds_ratio,
+                                               m->d_topn_beam);
     PSB_LAUNCH_CHECK();
     return PSB_OK;
 }
@@ -1570,6 +1282,9 @@ int psb_launch_ptm_batch(psb_batch_t *b, const float *d_feats, const int32_t *ut
     tabs.grp_base = reinterpret_cast<const long long *>(b->d_tab + n32);
     const long long *d_warp_base = tabs.grp_base + n_groups;
 
+    // Top-N kernels, by model shape: the tensor-core filter where psb_tc_usable allows it; else, for semi-continuous
+    // models with one codebook and n_density in {64, 128, 256}, the split path (semi_dist / semi_scan); else one scan
+    // per stream length (launch_topn).
     const bool use_tc = !semi && psb_tc_usable(b);
     if (b->have_ev) PSB_CUDA(cudaEventRecord(b->ev[0], b->stream));
     if (!use_tc) {
@@ -1584,7 +1299,7 @@ int psb_launch_ptm_batch(psb_batch_t *b, const float *d_feats, const int32_t *ut
     }
     if (b->have_ev) PSB_CUDA(cudaEventRecord(b->ev[1], b->stream));
     // semi-continuous: distances out of the time loop, one warp per (utterance, stream)
-    const bool semi_split = semi && !m->fixed_point && m->n_mgau == 1 && b->topn_variant != 0 && m->n_density <= 256 &&
+    const bool semi_split = semi && !m->fixed_point && m->n_mgau == 1 &&
                             (m->n_density == 64 || m->n_density == 128 || m->n_density == 256);
     if (use_tc) {
         // no recurrence over time: tensor-core filter, exact rescoring of the survivors, tie fix-up (psb_ptm_tc.cu)
@@ -1651,14 +1366,15 @@ int psb_launch_ptm_batch(psb_batch_t *b, const float *d_feats, const int32_t *ut
         }
     }
     if (b->have_ev) PSB_CUDA(cudaEventRecord(b->ev[2], b->stream));
+    // Senone kernels: 8-bit weights take the 16x2 kernel (four senones per thread) when (TOPN - 1) times the largest
+    // add-table entry stays below SEN_BIAS, else -- and for 4-bit weights -- the scalar kernel.
     if (semi) {
         size_t smem = (size_t)K * 32 + PSB_LOGADD8_N + 16;
         PSB_REQUIRE(K <= 512, "semi_senone_kernel handles at most 512 streams (got %d)", K);
         const int threads = 256;
         dim3 grid((m->n_sen + threads - 1) / threads, (unsigned)total);
         PSB_REQUIRE(total <= 65535LL * 32768, "too many frames for one launch");
-        if (!m->mixw_4bit && b->topn_variant != 0 && (TOPN - 1) * m->logadd8_max < SEN_BIAS && m->mixw_stride % 4 == 0 &&
-            m->n_feat <= PSB_MAX_FEAT)
+        if (!m->mixw_4bit && (TOPN - 1) * m->logadd8_max < SEN_BIAS && m->mixw_stride % 4 == 0 && m->n_feat <= PSB_MAX_FEAT)
             semi_senone4_kernel<<<(unsigned)total, 512, 0, b->stream>>>(b->d_topn, m->d_mixw, m->d_logadd8, d_senscr, m->n_sen,
                                                                       m->n_feat, m->n_density, m->mixw_stride);
         else if (m->mixw_4bit)
@@ -1680,7 +1396,8 @@ int psb_launch_ptm_batch(psb_batch_t *b, const float *d_feats, const int32_t *ut
                 b->d_topn, m->d_mixw, m->d_mixw_cb, m->d_sen2cb, m->d_logadd8, d_senscr, m->n_sen, m->n_feat,
                 m->n_density, K, m->mixw_stride);
         }
-        else if (b->topn_variant == 0 || (TOPN - 1) * m->logadd8_max >= SEN_BIAS) {
+        else if ((TOPN - 1) * m->logadd8_max >= SEN_BIAS) {
+            // the 16x2 arithmetic's bias would not cover the add table (a -logbase closer to 1 than the default)
             PSB_CUDA(cudaFuncSetAttribute(ptm_senone_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
             ptm_senone_kernel<false><<<(unsigned)total, 512, smem, b->stream>>>(
                 b->d_topn, m->d_mixw, m->d_mixw_cb, m->d_sen2cb, m->d_logadd8, d_senscr, m->n_sen, m->n_feat,
@@ -1693,21 +1410,8 @@ int psb_launch_ptm_batch(psb_batch_t *b, const float *d_feats, const int32_t *ut
             // at least 256 threads (log-add table staging) and one thread per (codebook, stream) pair
             const int threads = std::min(512, std::max(std::max(256, roundup(K, 32)), roundup((n_quads + iters - 1) / iters, 32)));
             const size_t smem4 = smem + 8 + (size_t)K * 16;
-            // experiment, off by default: measured 30.8 ms vs 18.9 ms per 998 k frames -- the 4 KB two-index table trades two
-            // mostly-broadcast byte reads for one read that bank-conflicts across 1024 words (bit-identical either way)
-            static const bool use_tab2 = getenv("PSB_SENONE_TAB2") && atoi(getenv("PSB_SENONE_TAB2")) == 1;
-            if (m->logadd8_zero_from <= 31 && use_tab2) {
-                const size_t smem5 = smem4 + 16 + 4096;
-                PSB_CUDA(cudaFuncSetAttribute(ptm_senone4_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem5));
-                ptm_senone4_kernel<true><<<(unsigned)total, threads, smem5, b->stream>>>(
-                    b->d_topn, m->d_mixw, m->d_sen2cb, m->d_quadcb, m->d_bsen, m->n_bsen, m->d_logadd8, d_senscr, m->n_sen,
-                    m->n_feat, m->n_density, K, m->mixw_stride);
-                PSB_LAUNCH_CHECK();
-                if (b->have_ev) PSB_CUDA(cudaEventRecord(b->ev[3], b->stream));
-                return PSB_OK;
-            }
-            PSB_CUDA(cudaFuncSetAttribute(ptm_senone4_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem4));
-            ptm_senone4_kernel<false><<<(unsigned)total, threads, smem4, b->stream>>>(
+            PSB_CUDA(cudaFuncSetAttribute(ptm_senone4_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem4));
+            ptm_senone4_kernel<<<(unsigned)total, threads, smem4, b->stream>>>(
                 b->d_topn, m->d_mixw, m->d_sen2cb, m->d_quadcb, m->d_bsen, m->n_bsen, m->d_logadd8, d_senscr, m->n_sen,
                 m->n_feat, m->n_density, K, m->mixw_stride);
         }

@@ -16,13 +16,13 @@
 //      `d >= (float)worst` holds -- and can never be evicted.  The list is then exactly those four
 //      in descending order, whatever the seeds were.  Only when two of the five best integer scores
 //      coincide do the order-dependent rules (`>=` shifting, strict `>` in eval_topn,
-//      skip-if-listed) matter; those frames are flagged and redone by ptm_fixup_kernel, which
+//      skip-if-listed) matter; those frames are flagged and redone by ptm_fixup_warp_kernel, which
 //      replays the reference's loop literally with the previous frame's list as seeds.
 //  (2) The five best can be found without computing 256 exact distances.  With y = x - m (m = the
 //      codebook's mean centre) the exponent d = det - sum_j v_j (y_j - mu'_j)^2 is the inner product
 //      of X = (y_j^2, y_j, 1) with W_c = (-v_cj, 2 v_cj mu'_cj, det_c - sum_j v_cj mu'_cj^2): one
-//      [frames x 32] x [32 x n_density] TF32 GEMM per pair on the tensor cores (mma.sync m16n8k8;
-//      the operands are rounded to TF32 once, on the host for W).  Its result a_c differs from the
+//      [frames x 32] x [32 x n_density] TF32 GEMM per pair on the tensor cores (tcgen05.mma, three
+//      products of high and low TF32 halves; W is split on the host).  Its result a_c differs from the
 //      reference's float d_c by at most eps = ERR * (sum_j Amax_j y_j^2 + Bmax_j |y_j| + Cmax), a
 //      bound every row computes for itself (Amax/Bmax/Cmax: per-pair maxima of |W| entries).  Five
 //      distinct codewords with a_c >= L0 (the four per-lane row maxima of the accumulator fragment
@@ -33,11 +33,9 @@
 //      them (anything else has d_c < d(4) - 1, i.e. a strictly smaller integer score): E (five to
 //      seven codewords) is what gets the reference's exact float arithmetic.
 //
-// The exact stage keeps the warp-uniform record stream of the old kernels: lane = frame (32
-// consecutive frames of the batch per warp), the warp walks the UNION of its lanes' E sets pair by
-// pair with the packed FADD2/FMUL2 distance (gau_dist2) and each lane keeps the five best of its
-// own set.  A row whose candidate list overflows its shared-memory slots falls back to E = C; a warp
-// whose rows agree on nothing degrades towards the dense scan, never below it.
+// The exact stage: a row the filter values leave in doubt goes on a work list that ptm_tc_exact_kernel
+// rescores, one thread per row, with the reference's float arithmetic over its candidates (over all
+// codewords when the row's candidate list overflowed its shared-memory slots).
 //
 // Nothing here is approximate in its output: tests/test_gpu_parity.py compares every record with the
 // oracle's lists, PSB_TC_CHECK=1 makes the filter kernel measure max |a_c - d_c| / eps on the device.
@@ -52,7 +50,6 @@ namespace {
 
 constexpr int TC_ROWS = 128;          // frames per CTA (4 warps x 2 m-tiles x 16 rows)
 constexpr int TC_K = 32;              // GEMM depth: 2 * FL + 1 <= 32
-constexpr int TC_XS = 36;             // row pitch of the X tile in floats (conflict-free fragment loads)
 constexpr int TC_CAP = 18;            // candidate slots per row: the row's X storage, 144 B / 8 B
 constexpr float TC_ERR = 1.0f / 262144.f;  // 2^-18 of the magnitude sum S: 3 x TF32 leaves 3 * 2^-22 per product, the rest is
                                            // room for the tensor core's fp32 accumulation (<= 2^-23 per step assumed, 12 steps per
@@ -63,13 +60,6 @@ __device__ __forceinline__ float to_tf32(float x)
     unsigned r;
     asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
     return __uint_as_float(r);
-}
-
-__device__ __forceinline__ void mma_tf32(float (&d)[4], const unsigned (&a)[4], float b0, float b1)
-{
-    asm volatile("mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-                 : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
-                 : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(__float_as_uint(b0)), "r"(__float_as_uint(b1)));
 }
 
 struct Top5 {
@@ -103,273 +93,8 @@ __device__ __forceinline__ void top5_insert(Top5 &t, int s, int c)
     if (t.n < 5) ++t.n;
 }
 
-// Filter + resolution for one (pair, 128-frame tile).
-//   wfrag   [K][2][NT][4][32] float2   W (high, then low TF32 halves) in mma B-fragment order:
-//                                      b0 = W[8 ks + t][8 n + g], b1 = W[8 ks + t + 4][8 n + g]
-//   cen     [K][16]                    centre m
-//   bnd     [K][32]                    Amax[FL], Bmax[FL], Cmax at [2 FL]
-//   rec     scalar records {det, mu0, v0, ...} of the model (exact distances of ambiguous rows, read through L1/L2)
-//   flags   [K][flag_words]            bit (row & 31) of word row >> 5: frame must be redone by the fix-up
-//   check   (debug) float[2]: max over everything of |a_c - d_c| / eps, and of the candidate count
-//   stats   (debug) unsigned long long[4]: rows, rows resolved from the filter alone, exact distances, tie flags
-template <int FL, int NT, bool CHECK>
-__global__ void __launch_bounds__(TC_ROWS, 4)
-ptm_tc_kernel(const float *__restrict__ feats, long long total, int D, const int32_t *__restrict__ featoff,
-              const int32_t *__restrict__ klist, const float2 *__restrict__ wfrag, const float *__restrict__ cen,
-              const float *__restrict__ bnd, const float *__restrict__ rec, const size_t *__restrict__ rec_off,
-              int4 *__restrict__ out, unsigned *__restrict__ flags, long long flag_words, int K, int n_feat,
-              float *__restrict__ check, unsigned long long *__restrict__ stats)
-{
-    constexpr int ND = NT * 8;
-    constexpr int RF = (1 + 2 * FL + 3) / 4 * 4;
-    constexpr unsigned FULL = 0xffffffffu;
-    static_assert(2 * FL + 1 <= TC_K, "stream too long for one 32-deep GEMM");
-    extern __shared__ __align__(16) unsigned char tc_smem[];
-    float2 *wf = reinterpret_cast<float2 *>(tc_smem);                                   // [NT][4][32]: high halves of W
-    float *xs = reinterpret_cast<float *>(tc_smem + (size_t)NT * 4 * 32 * 8);           // [128][36]; later the candidate lists
-    unsigned *masks = reinterpret_cast<unsigned *>(xs + TC_ROWS * TC_XS);               // [128][8]
-    int *cnt = reinterpret_cast<int *>(masks + TC_ROWS * 8);                            // [128]
-    float *epsr = reinterpret_cast<float *>(cnt + TC_ROWS);                             // [128]
-
-    const int k = klist[blockIdx.y];
-    const int f = k % n_feat;
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const long long row = (long long)blockIdx.x * TC_ROWS + tid;
-    const bool valid = row < total;
-
-    // ---- stage W (both halves), build this thread's X row (fp32: split into TF32 halves at fragment load) ----
-    {
-        const float4 *src = reinterpret_cast<const float4 *>(wfrag + (size_t)k * 2 * NT * 4 * 32);
-        float4 *dst = reinterpret_cast<float4 *>(wf);
-        for (int i = tid; i < NT * 4 * 32 / 2; i += TC_ROWS) dst[i] = src[i];
-    }
-    float x[FL];
-    {
-        const float *p = feats + (valid ? row : 0) * D + featoff[f];
-        const float *m = cen + (size_t)k * 16, *bb = bnd + (size_t)k * 32;
-        float S = bb[2 * FL];
-        float *xr = xs + tid * TC_XS;
-#pragma unroll
-        for (int j = 0; j < FL; ++j) {
-            x[j] = valid ? p[j] : 0.f;
-            const float y = __fsub_rn(x[j], m[j]);
-            const float y2 = __fmul_rn(y, y);
-            xr[j] = y2;
-            xr[FL + j] = y;
-            S = __fadd_ru(S, __fmul_ru(bb[j], y2));
-            S = __fadd_ru(S, __fmul_ru(bb[FL + j], fabsf(y)));
-        }
-        xr[2 * FL] = 1.0f;
-#pragma unroll
-        for (int j = 2 * FL + 1; j < TC_K; ++j) xr[j] = 0.f;
-        epsr[tid] = __fadd_ru(__fmul_ru(S, TC_ERR), 2.0f);
-        cnt[tid] = 0;
-#pragma unroll
-        for (int w = 0; w < 8; ++w) masks[tid * 8 + w] = 0u;
-    }
-    __syncthreads();
-
-    // ---- 3 x TF32 GEMM (lo*hi + hi*lo + hi*hi) of this warp's 32 rows against all codewords, 16 rows at a time.
-    // The accumulators are never held for all codewords at once: a first sweep over chunks of CH n-tiles keeps only
-    // the row maxima that give the threshold, a second sweep recomputes the same chunks (bit-identical: same
-    // instructions, same order) and extracts the few columns above it.  The tensor pipe has the room (< 10 % busy
-    // with one sweep); 40 accumulator registers instead of 128 double the resident warps. ----
-    constexpr int CH = NT <= 8 ? NT / 2 : 8;             // at least two chunks: the two half maxima per lane come from different chunks
-    const int g = lane >> 2, t = lane & 3;
-    uint2 *lists = reinterpret_cast<uint2 *>(xs);            // row r: slots at (r * TC_XS floats) .. + TC_CAP
-    const float2 *wlo = wfrag + ((size_t)k * 2 + 1) * NT * 4 * 32;      // low halves of W: from L1 / L2, same fragment order
-#pragma unroll 1
-    for (int mt = 0; mt < 2; ++mt) {
-        unsigned ah[4][4], al[4][4];
-        {
-            const float *xa = xs + (warp * 32 + mt * 16 + g) * TC_XS, *xb = xa + 8 * TC_XS;
-#pragma unroll
-            for (int ks = 0; ks < 4; ++ks) {
-                const float v[4] = {xa[8 * ks + t], xb[8 * ks + t], xa[8 * ks + t + 4], xb[8 * ks + t + 4]};
-#pragma unroll
-                for (int q = 0; q < 4; ++q) {
-                    const float h = to_tf32(v[q]);
-                    ah[ks][q] = __float_as_uint(h);
-                    al[ks][q] = __float_as_uint(to_tf32(__fsub_rn(v[q], h)));
-                }
-            }
-        }
-        __syncwarp();                                        // this m-tile's X rows now become their candidate lists
-        auto chunk = [&](int n0, float (&acc)[CH][4]) {
-#pragma unroll
-            for (int i = 0; i < CH; ++i) {
-                const int n = n0 + i;
-                acc[i][0] = acc[i][1] = acc[i][2] = acc[i][3] = 0.f;
-#pragma unroll
-                for (int ks = 0; ks < 4; ++ks) {             // the small cross terms first
-                    const float2 bh = wf[(n * 4 + ks) * 32 + lane], bl = __ldg(wlo + (n * 4 + ks) * 32 + lane);
-                    mma_tf32(acc[i], al[ks], bh.x, bh.y);
-                    mma_tf32(acc[i], ah[ks], bl.x, bl.y);
-                }
-#pragma unroll
-                for (int ks = 0; ks < 4; ++ks) {
-                    const float2 bh = wf[(n * 4 + ks) * 32 + lane];
-                    mma_tf32(acc[i], ah[ks], bh.x, bh.y);
-                }
-            }
-        };
-        // rows g (acc[.][0..1]) and g + 8 (acc[.][2..3]) of this m-tile: the lane's two half maxima each
-        const int r0 = warp * 32 + mt * 16 + g, r1 = r0 + 8;
-        float h00 = -INFINITY, h01 = -INFINITY, h10 = -INFINITY, h11 = -INFINITY;
-#pragma unroll 1
-        for (int n0 = 0; n0 < NT; n0 += CH) {
-            float acc[CH][4];
-            chunk(n0, acc);
-            float a = -INFINITY, b = -INFINITY;
-#pragma unroll
-            for (int i = 0; i < CH; ++i) { a = fmaxf(a, fmaxf(acc[i][0], acc[i][1])); b = fmaxf(b, fmaxf(acc[i][2], acc[i][3])); }
-            if (n0 < NT / 2) { h00 = fmaxf(h00, a); h10 = fmaxf(h10, b); }
-            else { h01 = fmaxf(h01, a); h11 = fmaxf(h11, b); }
-        }
-        float hi0 = fmaxf(h00, h01), lo0 = fminf(h00, h01), hi1 = fmaxf(h10, h11), lo1 = fminf(h10, h11);
-        // five distinct columns >= L0: the quad's four lane maxima and the best runner-up half maximum
-        hi0 = fminf(hi0, __shfl_xor_sync(FULL, hi0, 1)); hi0 = fminf(hi0, __shfl_xor_sync(FULL, hi0, 2));
-        lo0 = fmaxf(lo0, __shfl_xor_sync(FULL, lo0, 1)); lo0 = fmaxf(lo0, __shfl_xor_sync(FULL, lo0, 2));
-        hi1 = fminf(hi1, __shfl_xor_sync(FULL, hi1, 1)); hi1 = fminf(hi1, __shfl_xor_sync(FULL, hi1, 2));
-        lo1 = fmaxf(lo1, __shfl_xor_sync(FULL, lo1, 1)); lo1 = fmaxf(lo1, __shfl_xor_sync(FULL, lo1, 2));
-        const float e0 = epsr[r0], e1 = epsr[r1];
-        // L' = floor(L0 - eps) - 1, candidates: a_c >= L' - eps; every step rounded towards -inf
-        const float thr0 = __fsub_rd(__fsub_rd(floorf(__fsub_rd(fminf(hi0, lo0), e0)), 1.0f), e0);
-        const float thr1 = __fsub_rd(__fsub_rd(floorf(__fsub_rd(fminf(hi1, lo1), e1)), 1.0f), e1);
-        const float thr_min = fminf(thr0, thr1);
-        float worst = 0.f;
-#pragma unroll 1
-        for (int n0 = 0; n0 < NT; n0 += CH) {
-            float acc[CH][4];
-            chunk(n0, acc);
-#pragma unroll
-            for (int i = 0; i < CH; ++i) {
-                if (fmaxf(fmaxf(acc[i][0], acc[i][1]), fmaxf(acc[i][2], acc[i][3])) < thr_min) continue;
-#pragma unroll
-                for (int q = 0; q < 4; ++q) {
-                    const float a = acc[i][q];
-                    if (a >= ((q & 2) ? thr1 : thr0)) {
-                        const int rr = (q & 2) ? r1 : r0, col = 8 * (n0 + i) + 2 * t + (q & 1);
-                        const int slot = atomicAdd(&cnt[rr], 1);
-                        if (slot < TC_CAP) lists[(size_t)rr * (TC_XS / 2) + slot] = make_uint2(__float_as_uint(a), (unsigned)col);
-                        atomicOr(&masks[rr * 8 + (col >> 5)], 1u << (col & 31));
-                    }
-                }
-            }
-            if (CHECK) {
-                // exact distances of every column this lane holds (debug only): |a - d| / eps
-                const float *rc = rec + rec_off[k];
-                for (int i = 0; i < CH; ++i)
-                    for (int q = 0; q < 4; ++q) {
-                        const int rr = (q & 2) ? r1 : r0, col = 8 * (n0 + i) + 2 * t + (q & 1);
-                        const long long grow = (long long)blockIdx.x * TC_ROWS + rr;
-                        if (grow >= total) continue;
-                        const float *px = feats + grow * D + featoff[f];
-                        const float *r = rc + (size_t)col * RF;
-                        float d = r[0];
-                        for (int j = 0; j < FL; ++j) {
-                            const float df = __fsub_rn(px[j], r[1 + 2 * j]);
-                            d = __fsub_rn(d, __fmul_rn(__fmul_rn(df, df), r[2 + 2 * j]));
-                        }
-                        worst = fmaxf(worst, __fdividef(fabsf(acc[i][q] - d), epsr[rr]));
-                    }
-            }
-        }
-        if (CHECK) atomicMax(reinterpret_cast<int *>(check), __float_as_int(worst));     // non-negative floats order like ints
-    }
-    __syncthreads();
-    if (!valid) return;
-
-    // ---- one thread per row: the record straight from the filter values when they leave no doubt ----
-    const int n = cnt[tid];
-    const float ee = epsr[tid];
-    if (CHECK) atomicMax(reinterpret_cast<int *>(check) + 1, n);
-    Top5 top;
-    top.n = 0; top.c = 0u; top.c4 = 0;
-#pragma unroll
-    for (int j = 0; j < 5; ++j) top.s[j] = INT_MIN;
-    bool certain = n <= TC_CAP;
-    if (certain) {
-        // the five largest a_c with their codewords (the list holds every a_c >= thr, at least five)
-        const uint2 *L = lists + (size_t)tid * (TC_XS / 2);
-        float a[5] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY, -INFINITY};
-        int c[5] = {0, 0, 0, 0, 0};
-        for (int i = 0; i < n; ++i) {
-            float v = __uint_as_float(L[i].x);
-            int cv = (int)L[i].y;
-#pragma unroll
-            for (int j = 0; j < 5; ++j)
-                if (v > a[j]) { const float tv = a[j]; const int tc = c[j]; a[j] = v; c[j] = cv; v = tv; cv = tc; }
-        }
-        // order and distinctness of the truncated scores: neighbours more than 2 eps + 1 apart, everything
-        // safely negative (truncation is towards zero); s >> 10 of the four best: the same at both ends of
-        // [a - eps, a + eps]
-        const float gap = __fadd_ru(__fadd_ru(ee, ee), 1.0f);
-        int qv[4];
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-            certain &= __fsub_rd(a[j], a[j + 1]) > gap;
-            const int lo = __float2int_ru(__fsub_rd(a[j], ee)), hi = __float2int_ru(__fadd_ru(a[j], ee));
-            certain &= (lo >> PSB_SENSCR_SHIFT) == (hi >> PSB_SENSCR_SHIFT);
-            qv[j] = lo >> PSB_SENSCR_SHIFT;
-        }
-        certain &= __fadd_ru(a[0], ee) < -2.0f && a[4] > -2.0e9f;
-        if (certain) {
-            unsigned cb = 0, eb = 0;
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-                int ev = qv[0] - qv[j];
-                ev = ev > 255 ? 255 : ev;
-                cb |= (unsigned)c[j] << (8 * j);
-                eb |= (unsigned)ev << (8 * j);
-            }
-            out[row * K + k] = make_int4(qv[0], (int)cb, (int)eb, 0);
-            if (CHECK) { atomicAdd(stats, 1ull); atomicAdd(stats + 1, 1ull); }
-            return;
-        }
-    }
-    // ---- doubt: the reference's exact arithmetic for this row's candidates (few rows, few codewords each) ----
-    {
-        const float *rc = rec + rec_off[k];
-        int n_exact = 0;
-        auto exact = [&](int cw) {
-            const float4 *r4 = reinterpret_cast<const float4 *>(rc + (size_t)cw * RF);
-            const float d = gau_dist<FL>(r4, x);
-            top5_insert(top, f2i_clamped(d), cw);
-            ++n_exact;
-        };
-        if (n <= TC_CAP) {
-            const uint2 *L = lists + (size_t)tid * (TC_XS / 2);
-            // ascending codeword order is not needed: ties are redone by the fix-up
-            for (int i = 0; i < n; ++i) exact((int)L[i].y);
-        }
-        else {
-            for (int w = 0; w < ND / 32; ++w) {
-                unsigned bits = masks[tid * 8 + w];
-                while (bits) {
-                    const int b = __ffs(bits) - 1;
-                    bits &= bits - 1;
-                    exact(w * 32 + b);
-                }
-            }
-        }
-        const bool distinct = top.n >= 5 && top.s[0] > top.s[1] && top.s[1] > top.s[2] && top.s[2] > top.s[3] && top.s[3] > top.s[4];
-        const int tp = top.s[0] >> PSB_SENSCR_SHIFT;
-        unsigned eb = 0;
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-            int ev = tp - (top.s[j] >> PSB_SENSCR_SHIFT);
-            ev = ev > 255 ? 255 : ev;
-            eb |= (unsigned)ev << (8 * j);
-        }
-        out[row * K + k] = make_int4(tp, (int)top.c, (int)eb, 0);
-        if (!distinct) atomicOr(&flags[(size_t)k * flag_words + (row >> 5)], 1u << (row & 31));
-        if (CHECK) { atomicAdd(stats, 1ull); atomicAdd(stats + 2, (unsigned long long)n_exact); if (!distinct) atomicAdd(stats + 3, 1ull); }
-    }
-}
-
 // ---------------------------------------------------------------------------------------
-// The same filter on the 5th-generation tensor cores (tcgen05): the legacy mma.sync path above tops out
+// The filter on the 5th-generation tensor cores (tcgen05): mma.sync tops out
 // near 290 TFLOP/s of TF32 (8 cycles per m16n8k8 and sub-core), which makes the 3 x TF32 GEMM -- 6.2 TFLOP
 // per 10^6-frame batch -- the longest stage.  Here one elected thread issues twelve
 // tcgen05.mma.cta_group::1.kind::tf32 (M 128 frames x N n_density x K 8; lo*hi, hi*lo, hi*hi over four
@@ -453,13 +178,16 @@ __device__ __forceinline__ void mbar_wait_parity(uint64_t *bar, unsigned parity)
         : "memory");
 }
 
+// Filter + resolution for a pair's tiles of 128 frames.
 //   wumma   [K][2][8][ND][4] float   W halves (high, low) in the canonical K-major layout: chunk kc holds k = 4 kc .. 4 kc + 3
-// SPLIT = 2: two threads per frame (256 threads per CTA), each sweeping half of the columns of the SAME accumulator row
-// (warps w and w + 4 own the same 32 TMEM lanes): the accumulator sweeps are the longest serial stretch of a tile and the
-// tensor memory (two 256-column accumulators per SM) caps the CTAs at two, so this is the way to put sixteen warps on
-// an SM.  The halves meet twice: eight group maxima per row, and the two candidate sub-lists that thread 0 of the pair resolves.
-template <int FL, int ND, int SPLIT, bool CHECK>
-__global__ void __launch_bounds__(TC_ROWS * SPLIT, 2)
+//   cen     [K][16]                    centre m
+//   bnd     [K][32]                    Amax[FL], Bmax[FL], Cmax at [2 FL]
+//   rec     scalar records {det, mu0, v0, ...} of the model (exact distances of ambiguous rows, read through L1/L2)
+//   flags   [K][flag_words]            bit (row & 31) of word row >> 5: frame must be redone by the fix-up
+//   check   (debug) float[2]: max over everything of |a_c - d_c| / eps, and of the candidate count
+//   stats   (debug) unsigned long long[4]: rows, rows resolved from the filter alone, exact distances, tie flags
+template <int FL, int ND, bool CHECK>
+__global__ void __launch_bounds__(TC_ROWS, 2)
 ptm_tc5_kernel(const float *__restrict__ feats, long long total, int D, const int32_t *__restrict__ featoff,
                const int32_t *__restrict__ klist, const float *__restrict__ wumma, const float *__restrict__ cen,
                const float *__restrict__ bnd, const float *__restrict__ rec, const size_t *__restrict__ rec_off,
@@ -469,23 +197,17 @@ ptm_tc5_kernel(const float *__restrict__ feats, long long total, int D, const in
 {
     constexpr int RF = (1 + 2 * FL + 3) / 4 * 4;
     constexpr int GW = ND / 8;                           // columns per maximum group: 8 groups per row
-    constexpr int NT_ = TC_ROWS * SPLIT;                 // threads
-    constexpr int NDH = ND / SPLIT;                      // columns per thread
-    constexpr int CAPH = SPLIT == 1 ? TC_CAP : 12;       // candidate slots per thread
-    constexpr int SD = 32 / SPLIT;                       // columns staged at a time
-    static_assert(2 * FL + 1 <= TC_K && ND % 32 == 0 && ND <= 256 && NDH % 64 == 0 && (SPLIT == 1 || SPLIT == 2), "shape");
+    static_assert(2 * FL + 1 <= TC_K && ND % 32 == 0 && ND <= 256 && ND % 64 == 0, "shape");
     extern __shared__ __align__(128) unsigned char t5_smem[];
     float *sW = reinterpret_cast<float *>(t5_smem);                                   // [2][8][ND][4]
     float *sX = sW + 2 * 8 * ND * 4;                                                  // [2][8][128][4]; after the MMA: lists + staging
     // thread-private and transposed ([slot][thread]: conflict-free): candidate values, candidate columns, one 32-column slab
-    float *Lv = sX;                                                                   // [CAPH][threads]
-    unsigned char *Lc = reinterpret_cast<unsigned char *>(Lv + CAPH * NT_);           // [CAPH][threads]
-    float *stage = reinterpret_cast<float *>(Lc + ((CAPH * NT_ + 15) & ~15));         // [SD][threads]
-    static_assert(CAPH * NT_ * 5 + 16 + SD * NT_ * 4 <= 2 * 8 * TC_ROWS * 16, "lists + staging must fit the X tile");
+    float *Lv = sX;                                                                   // [TC_CAP][TC_ROWS]
+    unsigned char *Lc = reinterpret_cast<unsigned char *>(Lv + TC_CAP * TC_ROWS);     // [TC_CAP][TC_ROWS]
+    float *stage = reinterpret_cast<float *>(Lc + ((TC_CAP * TC_ROWS + 15) & ~15));   // [32][TC_ROWS]
+    static_assert(TC_CAP * TC_ROWS * 5 + 16 + 32 * TC_ROWS * 4 <= 2 * 8 * TC_ROWS * 16, "lists + staging must fit the X tile");
     __shared__ __align__(8) uint64_t mma_done;
     __shared__ unsigned tmem_base_s;
-    __shared__ float gmx[SPLIT == 1 ? 1 : TC_ROWS * 8];                               // SPLIT = 2: the row's eight group maxima
-    __shared__ int cnt_s[SPLIT == 1 ? 1 : 2 * TC_ROWS];                               // SPLIT = 2: candidates per half
 
     // grid: x = pair (fastest), y = group of tiles: CTAs that run together read the SAME frames for different pairs, so
     // the feature rows come out of L2 (with tiles fastest every pair re-read the whole feature matrix from HBM: 23 GB
@@ -493,7 +215,7 @@ ptm_tc5_kernel(const float *__restrict__ feats, long long total, int D, const in
     const int k = klist[blockIdx.x];
     const int f = k % n_feat;
     const int tid = threadIdx.x, warp = tid >> 5;
-    const int r = tid & (TC_ROWS - 1), half = tid / TC_ROWS;          // this thread's frame of the tile and its half of the columns
+    const int r = tid;                                   // this thread's frame of the tile
 
     if (warp == 0) {                                     // 256 (or fewer) TMEM columns for the accumulator
         asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"((unsigned)__cvta_generic_to_shared(&tmem_base_s)),
@@ -507,7 +229,7 @@ ptm_tc5_kernel(const float *__restrict__ feats, long long total, int D, const in
     {
         const float4 *src = reinterpret_cast<const float4 *>(wumma + (size_t)k * 2 * 8 * ND * 4);
         float4 *dst = reinterpret_cast<float4 *>(sW);
-        for (int i = tid; i < 2 * 8 * ND; i += NT_) dst[i] = src[i];
+        for (int i = tid; i < 2 * 8 * ND; i += TC_ROWS) dst[i] = src[i];
     }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
@@ -551,7 +273,6 @@ ptm_tc5_kernel(const float *__restrict__ feats, long long total, int D, const in
             ee = __fadd_ru(__fmul_ru(S, TC_ERR), 2.0f);
 #pragma unroll
             for (int kc = 0; kc < 8; ++kc) {
-                if (SPLIT == 2 && (kc & 1) != half) continue;         // the pair shares the conversions and stores
                 float4 h, l;
                 h.x = to_tf32(v[4 * kc]); h.y = to_tf32(v[4 * kc + 1]); h.z = to_tf32(v[4 * kc + 2]); h.w = to_tf32(v[4 * kc + 3]);
                 l.x = to_tf32(__fsub_rn(v[4 * kc], h.x)); l.y = to_tf32(__fsub_rn(v[4 * kc + 1], h.y));
@@ -587,7 +308,7 @@ ptm_tc5_kernel(const float *__restrict__ feats, long long total, int D, const in
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
 
         // ---- this thread's row of the accumulator: group maxima, threshold, the columns above it ----
-        const unsigned trow = tmem_d + ((unsigned)((warp & 3) * 32) << 16) + (unsigned)(half * NDH);
+        const unsigned trow = tmem_d + ((unsigned)((warp & 3) * 32) << 16);
         float gm[8];
 #pragma unroll
         for (int i = 0; i < 8; ++i) gm[i] = -INFINITY;
@@ -598,7 +319,7 @@ ptm_tc5_kernel(const float *__restrict__ feats, long long total, int D, const in
 #pragma unroll
                 for (int i = 0; i < 8; ++i) m8[i] = fmaxf(fmaxf(v[i], v[i + 8]), fmaxf(v[i + 16], v[i + 24]));
                 const float mx = fmaxf(fmaxf(fmaxf(m8[0], m8[1]), fmaxf(m8[2], m8[3])), fmaxf(fmaxf(m8[4], m8[5]), fmaxf(m8[6], m8[7])));
-                const int gi = (half * NDH + c0) / GW;
+                const int gi = c0 / GW;
 #pragma unroll
                 for (int q = 0; q < 8; ++q)
                     if (q == gi) gm[q] = fmaxf(gm[q], mx);
@@ -610,7 +331,7 @@ ptm_tc5_kernel(const float *__restrict__ feats, long long total, int D, const in
                     float mx = v[s2 * GW];
 #pragma unroll
                     for (int i = 1; i < GW; ++i) mx = fmaxf(mx, v[s2 * GW + i]);
-                    const int gi = (half * NDH + c0) / GW + s2;
+                    const int gi = c0 / GW + s2;
 #pragma unroll
                     for (int q = 0; q < 8; ++q)
                         if (q == gi) gm[q] = fmaxf(gm[q], mx);
@@ -621,21 +342,14 @@ ptm_tc5_kernel(const float *__restrict__ feats, long long total, int D, const in
             float va[32], vb[32];
             tmem_ld32_issue(trow, va);
 #pragma unroll 1
-            for (int c0 = 0; c0 < NDH; c0 += 64) {
+            for (int c0 = 0; c0 < ND; c0 += 64) {
                 tmem_wait_ld_dep(va);
                 tmem_ld32_issue(trow + c0 + 32, vb);
                 maxima(c0, va);
                 tmem_wait_ld_dep(vb);
-                if (c0 + 64 < NDH) tmem_ld32_issue(trow + c0 + 64, va);
+                if (c0 + 64 < ND) tmem_ld32_issue(trow + c0 + 64, va);
                 maxima(c0 + 32, vb);
             }
-        }
-        if (SPLIT == 2) {                                 // the other half's group maxima
-#pragma unroll
-            for (int q = 0; q < 4; ++q) gmx[r * 8 + half * 4 + q] = gm[half * 4 + q];
-            __syncthreads();
-#pragma unroll
-            for (int q = 0; q < 8; ++q) gm[q] = gmx[r * 8 + q];
         }
         // five distinct columns >= L0: the fifth largest of the eight group maxima
         float L0;
@@ -662,24 +376,21 @@ ptm_tc5_kernel(const float *__restrict__ feats, long long total, int D, const in
             const unsigned hit_all = (h4[0] | h4[1]) | (h4[2] | h4[3]);
             if (__any_sync(0xffffffffu, hit_all != 0u)) {    // registers cannot be indexed by a run-time column: through shared memory
 #pragma unroll
-                for (int part = 0; part < SPLIT; ++part) {
-#pragma unroll
-                    for (int i = 0; i < SD; ++i) stage[i * NT_ + tid] = v[part * SD + i];
-                    unsigned hit = (hit_all >> (part * SD)) & (SD == 32 ? 0xffffffffu : ((1u << SD) - 1u));
-                    while (hit) {
-                        const int i = __ffs(hit) - 1;
-                        hit &= hit - 1;
-                        if (n < CAPH) {
-                            Lv[n * NT_ + tid] = stage[i * NT_ + tid];
-                            Lc[n * NT_ + tid] = (unsigned char)(half * NDH + c0 + part * SD + i);
-                        }
-                        ++n;
+                for (int i = 0; i < 32; ++i) stage[i * TC_ROWS + tid] = v[i];
+                unsigned hit = hit_all;
+                while (hit) {
+                    const int i = __ffs(hit) - 1;
+                    hit &= hit - 1;
+                    if (n < TC_CAP) {
+                        Lv[n * TC_ROWS + tid] = stage[i * TC_ROWS + tid];
+                        Lc[n * TC_ROWS + tid] = (unsigned char)(c0 + i);
                     }
+                    ++n;
                 }
             }
             if (CHECK && valid) {
                 for (int i = 0; i < 32; ++i) {
-                    const float *rp = rc + (size_t)(half * NDH + c0 + i) * RF;
+                    const float *rp = rc + (size_t)(c0 + i) * RF;
                     float d = rp[0];
                     for (int j = 0; j < FL; ++j) {
                         const float df = __fsub_rn(x[j], rp[1 + 2 * j]);
@@ -693,34 +404,26 @@ ptm_tc5_kernel(const float *__restrict__ feats, long long total, int D, const in
             float va[32], vb[32];
             tmem_ld32_issue(trow, va);
 #pragma unroll 1
-            for (int c0 = 0; c0 < NDH; c0 += 64) {
+            for (int c0 = 0; c0 < ND; c0 += 64) {
                 tmem_wait_ld_dep(va);
                 tmem_ld32_issue(trow + c0 + 32, vb);
                 collect(c0, va);
                 tmem_wait_ld_dep(vb);
-                if (c0 + 64 < NDH) tmem_ld32_issue(trow + c0 + 64, va);
+                if (c0 + 64 < ND) tmem_ld32_issue(trow + c0 + 64, va);
                 collect(c0 + 32, vb);
             }
         }
         asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-        // SPLIT = 2: thread 0 of the pair takes over with both sub-lists (own slots, then the partner's)
-        int n0 = n, n1 = 0;
-        if (SPLIT == 2) {
-            cnt_s[half * TC_ROWS + r] = n;
-            __syncthreads();
-            n0 = cnt_s[r]; n1 = cnt_s[TC_ROWS + r];
-        }
-        const bool listed = n0 <= CAPH && n1 <= CAPH && n0 + n1 >= 5 && n0 + n1 <= 20;
-        n = n0 + n1;
-        auto cand_v = [&](int i) { return i < n0 ? Lv[i * NT_ + r] : Lv[(i - n0) * NT_ + TC_ROWS + r]; };
-        auto cand_c = [&](int i) { return (int)(i < n0 ? Lc[i * NT_ + r] : Lc[(i - n0) * NT_ + TC_ROWS + r]); };
+        const bool listed = n >= 5 && n <= TC_CAP;
+        auto cand_v = [&](int i) { return Lv[i * TC_ROWS + r]; };
+        auto cand_c = [&](int i) { return (int)Lc[i * TC_ROWS + r]; };
         if (CHECK) {
             atomicMax(reinterpret_cast<int *>(check), __float_as_int(worst));
-            if (valid && half == 0) atomicMax(reinterpret_cast<int *>(check) + 1, n);
+            if (valid) atomicMax(reinterpret_cast<int *>(check) + 1, n);
         }
 
         // ---- the record straight from the filter values when they leave no doubt ----
-        if (valid && half == 0) {
+        if (valid) {
             bool certain = listed;
             if (certain) {
                 float a[5] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY, -INFINITY};
@@ -860,83 +563,13 @@ ptm_tc_exact_kernel(const float *__restrict__ feats, int D, const int32_t *__res
 
 // Frames whose five best scores tie: the reference's loop, literally (eval_topn ptm_mgau.c:88-136,
 // eval_cb :152-226), seeded with the previous frame's list -- the record the filter kernel (or this
-// thread, one frame earlier) wrote -- or with codewords 0..3 at the start of an utterance (:791-792).
-// One thread per (utterance, pair); flagged frames of a chain are visited in order.
-template <int FL>
-__global__ void __launch_bounds__(128)
-ptm_fixup_kernel(const float *__restrict__ feats, int D, const int32_t *__restrict__ featoff, const int32_t *__restrict__ utt_off,
-                 int n_utt, const float *__restrict__ rec, const size_t *__restrict__ rec_off, int4 *__restrict__ out,
-                 const unsigned *__restrict__ flags, long long flag_words, int K, int n_feat, int nd)
-{
-    constexpr int RF = (1 + 2 * FL + 3) / 4 * 4;
-    const long long id = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (id >= (long long)n_utt * K) return;
-    const int u = (int)(id / K), k = (int)(id % K);
-    const int f = k % n_feat;
-    const long long f0 = utt_off[u], f1 = utt_off[u + 1];
-    const unsigned *fl = flags + (size_t)k * flag_words;
-    const float *rc = rec + rec_off[k];
-    for (long long wd = f0 >> 5; wd <= (f1 - 1) >> 5 && f1 > f0; ++wd) {
-        unsigned bits = fl[wd];
-        while (bits) {
-            const int b = __ffs(bits) - 1;
-            bits &= bits - 1;
-            const long long row = wd * 32 + b;
-            if (row < f0 || row >= f1) continue;
-            const float *px = feats + row * D + featoff[f];
-            float x[FL];
-#pragma unroll
-            for (int j = 0; j < FL; ++j) x[j] = px[j];
-            const unsigned seeds = row == f0 ? 0x03020100u : (unsigned)out[(row - 1) * K + k].y;
-            int cw[4], sc[4];
-            for (int i = 0; i < 4; ++i) {                                   // eval_topn: stable, strict >
-                const int c = (seeds >> (8 * i)) & 0xff;
-                const float *r = rc + (size_t)c * RF;
-                float d = r[0];
-#pragma unroll
-                for (int j = 0; j < FL; ++j) {
-                    const float df = __fsub_rn(x[j], r[1 + 2 * j]);
-                    d = __fsub_rn(d, __fmul_rn(__fmul_rn(df, df), r[2 + 2 * j]));
-                }
-                const int s = f2i_clamped(d);
-                int j = i - 1;
-                while (j >= 0 && s > sc[j]) { sc[j + 1] = sc[j]; cw[j + 1] = cw[j]; --j; }
-                sc[j + 1] = s; cw[j + 1] = c;
-            }
-            for (int c = 0; c < nd; ++c) {                                  // eval_cb (early exit is result-neutral)
-                const float *r = rc + (size_t)c * RF;
-                float d = r[0];
-#pragma unroll
-                for (int j = 0; j < FL; ++j) {
-                    const float df = __fsub_rn(x[j], r[1 + 2 * j]);
-                    d = __fsub_rn(d, __fmul_rn(__fmul_rn(df, df), r[2 + 2 * j]));
-                }
-                if (!(d >= (float)sc[3])) continue;
-                if (cw[0] == c || cw[1] == c || cw[2] == c || cw[3] == c) continue;
-                const int s = f2i_clamped(d);
-                int kk = 3;
-                while (kk > 0 && s >= sc[kk - 1]) { sc[kk] = sc[kk - 1]; cw[kk] = cw[kk - 1]; --kk; }
-                sc[kk] = s; cw[kk] = c;
-            }
-            const int tp = sc[0] >> PSB_SENSCR_SHIFT;
-            unsigned cb = 0, eb = 0;
-            for (int j = 0; j < 4; ++j) {
-                int ev = tp - (sc[j] >> PSB_SENSCR_SHIFT);
-                ev = ev > 255 ? 255 : ev;
-                cb |= (unsigned)cw[j] << (8 * j);
-                eb |= (unsigned)ev << (8 * j);
-            }
-            out[row * K + k] = make_int4(tp, (int)cb, (int)eb, 0);
-        }
-    }
-}
-
-// The same fix-up with a WARP per (utterance, pair) chain: lanes = codewords (ND / 32 each), the flagged frames of the
+// warp, one frame earlier) wrote -- or with codewords 0..3 at the start of an utterance (:791-792).
+// One WARP per (utterance, pair) chain: lanes = codewords (ND / 32 each), the flagged frames of the
 // chain in order.  All distances of a frame in parallel, the four seeds fetched by shuffle, then the scan only visits --
 // in ascending codeword order -- the codewords whose distance reaches the seeds' worst score (ballots), each re-tested
 // against the list as it stands: eval_topn + eval_cb literally, like semi_scan_kernel does for semi-continuous models.
-// The thread-per-chain kernel above serialises 260 distances per flagged frame inside one lane (15 ms per 10^6 frames
-// at a 0.04 % tie rate); this one costs a few hundred warp instructions per flagged frame.
+// A thread per chain serialises 260 distances per flagged frame inside one lane (15 ms per 10^6 frames at a 0.04 % tie
+// rate); a warp costs a few hundred warp instructions per flagged frame.
 template <int FL, int NDW>
 __global__ void __launch_bounds__(128)
 ptm_fixup_warp_kernel(const float *__restrict__ feats, int D, const int32_t *__restrict__ featoff, const int32_t *__restrict__ utt_off,
@@ -1049,34 +682,7 @@ float round_tf32_host(float x)
     return r;
 }
 
-template <int FL, int NT>
-int launch_tc(psb_batch_t *b, const float *d_feats, long long total, const int32_t *d_klist, int n_k, const int32_t *d_featoff,
-              bool check)
-{
-    psb_model_t *m = b->m;
-    const size_t smem = (size_t)NT * 4 * 32 * 8 + (size_t)TC_ROWS * TC_XS * 4 + (size_t)TC_ROWS * 8 * 4 + TC_ROWS * 4 + TC_ROWS * 4;
-    const dim3 grid((unsigned)((total + TC_ROWS - 1) / TC_ROWS), (unsigned)n_k);
-    float *chk = b->d_tc_check;
-    unsigned long long *stats = reinterpret_cast<unsigned long long *>(b->d_tc_check + 4);
-    if (check) {
-        auto kern = ptm_tc_kernel<FL, NT, true>;
-        PSB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        kern<<<grid, TC_ROWS, smem, b->stream>>>(d_feats, total, m->sumlen, d_featoff, d_klist, reinterpret_cast<const float2 *>(m->d_tc_wfrag),
-                                                m->d_tc_cen, m->d_tc_bnd, m->d_rec, m->d_rec_off, b->d_topn, b->d_tc_flags,
-                                                (long long)b->tc_flag_words, m->K, m->n_feat, chk, stats);
-    }
-    else {
-        auto kern = ptm_tc_kernel<FL, NT, false>;
-        PSB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        kern<<<grid, TC_ROWS, smem, b->stream>>>(d_feats, total, m->sumlen, d_featoff, d_klist, reinterpret_cast<const float2 *>(m->d_tc_wfrag),
-                                                m->d_tc_cen, m->d_tc_bnd, m->d_rec, m->d_rec_off, b->d_topn, b->d_tc_flags,
-                                                (long long)b->tc_flag_words, m->K, m->n_feat, nullptr, nullptr);
-    }
-    PSB_LAUNCH_CHECK();
-    return PSB_OK;
-}
-
-template <int FL, int ND, int SPLIT>
+template <int FL, int ND>
 int launch_tc5(psb_batch_t *b, const float *d_feats, long long total, const int32_t *d_klist, int n_k, const int32_t *d_featoff,
                bool check)
 {
@@ -1091,16 +697,16 @@ int launch_tc5(psb_batch_t *b, const float *d_feats, long long total, const int3
     float *chk = b->d_tc_check;
     unsigned long long *stats = reinterpret_cast<unsigned long long *>(b->d_tc_check + 4);
     if (check) {
-        auto kern = ptm_tc5_kernel<FL, ND, SPLIT, true>;
+        auto kern = ptm_tc5_kernel<FL, ND, true>;
         PSB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        kern<<<grid, TC_ROWS * SPLIT, smem, b->stream>>>(d_feats, total, m->sumlen, d_featoff, d_klist, m->d_tc_wumma, m->d_tc_cen, m->d_tc_bnd,
+        kern<<<grid, TC_ROWS, smem, b->stream>>>(d_feats, total, m->sumlen, d_featoff, d_klist, m->d_tc_wumma, m->d_tc_cen, m->d_tc_bnd,
                                                 m->d_rec, m->d_rec_off, b->d_topn, b->d_tc_flags, (long long)b->tc_flag_words, m->K,
                                                 m->n_feat, tpc, b->d_tc_items, b->d_tc_nitems, b->tc_item_cap, chk, stats);
     }
     else {
-        auto kern = ptm_tc5_kernel<FL, ND, SPLIT, false>;
+        auto kern = ptm_tc5_kernel<FL, ND, false>;
         PSB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        kern<<<grid, TC_ROWS * SPLIT, smem, b->stream>>>(d_feats, total, m->sumlen, d_featoff, d_klist, m->d_tc_wumma, m->d_tc_cen, m->d_tc_bnd,
+        kern<<<grid, TC_ROWS, smem, b->stream>>>(d_feats, total, m->sumlen, d_featoff, d_klist, m->d_tc_wumma, m->d_tc_cen, m->d_tc_bnd,
                                                 m->d_rec, m->d_rec_off, b->d_topn, b->d_tc_flags, (long long)b->tc_flag_words, m->K,
                                                 m->n_feat, tpc, b->d_tc_items, b->d_tc_nitems, b->tc_item_cap, nullptr, nullptr);
     }
@@ -1128,9 +734,9 @@ int psb_tc_prepare(psb_model_t *m, const float *hm, const float *hv, const float
     if (m->n_density != 64 && m->n_density != 128 && m->n_density != 256) return PSB_OK;
     for (int f = 0; f < m->n_feat; ++f)
         if (m->featlen[f] != 13) return PSB_OK;              // the kernels are instantiated for 13-dimensional streams
-    const int nd = m->n_density, NT = nd / 8, FL = 13, K = m->K;
-    std::vector<float> wf((size_t)K * 2 * NT * 4 * 32 * 2, 0.f), cen((size_t)K * 16, 0.f), bnd((size_t)K * 32, 0.f);
-    std::vector<float> wu((size_t)K * 2 * 8 * nd * 4, 0.f);     // canonical K-major layout of the tcgen05 path: [half][chunk][n][4]
+    const int nd = m->n_density, FL = 13, K = m->K;
+    std::vector<float> cen((size_t)K * 16, 0.f), bnd((size_t)K * 32, 0.f);
+    std::vector<float> wu((size_t)K * 2 * 8 * nd * 4, 0.f);     // canonical K-major layout of the tcgen05 operand: [half][chunk][n][4]
     std::vector<double> W((size_t)TC_K * nd);
     for (int cb = 0; cb < m->n_mgau; ++cb)
         for (int f = 0; f < m->n_feat; ++f) {
@@ -1162,18 +768,6 @@ int psb_tc_prepare(psb_model_t *m, const float *hm, const float *hv, const float
             bb[2 * FL] = (float)(cmax * 1.0001);
             for (int j = 0; j < 2 * FL; ++j) bb[j] = std::nextafter(bb[j] * 1.0001f, INFINITY);
             // high and low TF32 halves of the fp32 value of every W entry: w = hi + lo + O(2^-22 w)
-            float *w = wf.data() + (size_t)k * 2 * NT * 4 * 32 * 2;
-            for (int n = 0; n < NT; ++n)
-                for (int ks = 0; ks < 4; ++ks)
-                    for (int lane = 0; lane < 32; ++lane) {
-                        const int g = lane >> 2, t = lane & 3;
-                        float *oh = w + ((size_t)(n * 4 + ks) * 32 + lane) * 2, *ol = oh + (size_t)NT * 4 * 32 * 2;
-                        for (int h = 0; h < 2; ++h) {
-                            const float v = (float)W[(size_t)(8 * ks + t + 4 * h) * nd + 8 * n + g];
-                            oh[h] = round_tf32_host(v);
-                            ol[h] = round_tf32_host(v - oh[h]);
-                        }
-                    }
             float *u = wu.data() + (size_t)k * 2 * 8 * nd * 4;
             for (int kk = 0; kk < TC_K; ++kk)
                 for (int q = 0; q < nd; ++q) {
@@ -1184,14 +778,12 @@ int psb_tc_prepare(psb_model_t *m, const float *hm, const float *hv, const float
             for (int i = 0; i < 32; ++i)
                 if (!std::isfinite(bb[i])) return PSB_OK;    // degenerate model: keep the scan kernels
         }
-    if (!m->d_tc_wfrag) {
+    if (!m->d_tc_wumma) {
         PSB_CUDA(cudaMalloc(&m->d_tc_wumma, wu.size() * sizeof(float)));
-        PSB_CUDA(cudaMalloc(&m->d_tc_wfrag, wf.size() * sizeof(float)));
         PSB_CUDA(cudaMalloc(&m->d_tc_cen, cen.size() * sizeof(float)));
         PSB_CUDA(cudaMalloc(&m->d_tc_bnd, bnd.size() * sizeof(float)));
     }
     PSB_CUDA(cudaMemcpy(m->d_tc_wumma, wu.data(), wu.size() * sizeof(float), cudaMemcpyHostToDevice));
-    PSB_CUDA(cudaMemcpy(m->d_tc_wfrag, wf.data(), wf.size() * sizeof(float), cudaMemcpyHostToDevice));
     PSB_CUDA(cudaMemcpy(m->d_tc_cen, cen.data(), cen.size() * sizeof(float), cudaMemcpyHostToDevice));
     PSB_CUDA(cudaMemcpy(m->d_tc_bnd, bnd.data(), bnd.size() * sizeof(float), cudaMemcpyHostToDevice));
     m->tc_ok = true;
@@ -1201,7 +793,7 @@ int psb_tc_prepare(psb_model_t *m, const float *hm, const float *hv, const float
 bool psb_tc_usable(const psb_batch_t *b)
 {
     const psb_model_t *m = b->m;
-    return m->tc_ok && m->ds_ratio == 1 && b->topn_variant >= 6;
+    return m->tc_ok && m->ds_ratio == 1 && !b->force_scan;
 }
 
 // Top-N records of a whole batch into b->d_topn (same format as the scan kernels write).
@@ -1243,41 +835,21 @@ int psb_launch_ptm_tc(psb_batch_t *b, const float *d_feats, const int32_t *utt_o
     PSB_CUDA(cudaMemsetAsync(b->d_tc_flags, 0, fw * m->K * 4, b->stream));
     PSB_CUDA(cudaMemcpyAsync(b->d_uttoff, utt_off, ((size_t)n_utt + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, b->stream));
     static const bool check = [] { const char *v = getenv("PSB_TC_CHECK"); return v && atoi(v) != 0; }();
-    static const bool legacy_mma = [] { const char *v = getenv("PSB_TC_IMPL"); return v && !strcmp(v, "mma"); }();   // default: tcgen05
     int rc;
-    if (legacy_mma)
-        switch (m->n_density) {
-        case 256: rc = launch_tc<13, 32>(b, d_feats, total, d_klist, m->K, d_featoff, check); break;
-        case 128: rc = launch_tc<13, 16>(b, d_feats, total, d_klist, m->K, d_featoff, check); break;
-        default: rc = launch_tc<13, 8>(b, d_feats, total, d_klist, m->K, d_featoff, check); break;
-        }
-    else
-    {
-        static const bool one_thread = [] { const char *v = getenv("PSB_TC_SPLIT"); return !(v && atoi(v) == 2); }();   // two threads per frame measured slower (DESIGN 4.15): 37.2 vs 30.7 ms
-        switch (m->n_density) {
-        case 256: rc = one_thread ? launch_tc5<13, 256, 1>(b, d_feats, total, d_klist, m->K, d_featoff, check)
-                                  : launch_tc5<13, 256, 2>(b, d_feats, total, d_klist, m->K, d_featoff, check); break;
-        case 128: rc = one_thread ? launch_tc5<13, 128, 1>(b, d_feats, total, d_klist, m->K, d_featoff, check)
-                                  : launch_tc5<13, 128, 2>(b, d_feats, total, d_klist, m->K, d_featoff, check); break;
-        default: rc = launch_tc5<13, 64, 1>(b, d_feats, total, d_klist, m->K, d_featoff, check); break;
-        }
+    switch (m->n_density) {
+    case 256: rc = launch_tc5<13, 256>(b, d_feats, total, d_klist, m->K, d_featoff, check); break;
+    case 128: rc = launch_tc5<13, 128>(b, d_feats, total, d_klist, m->K, d_featoff, check); break;
+    default: rc = launch_tc5<13, 64>(b, d_feats, total, d_klist, m->K, d_featoff, check); break;
     }
     if (rc) return rc;
     const long long chains = (long long)n_utt * m->K;
-    static const bool thread_fixup = [] { const char *v = getenv("PSB_TC_FIXUP"); return v && !strcmp(v, "thread"); }();
-    if (thread_fixup)
-        ptm_fixup_kernel<13><<<(unsigned)((chains + 127) / 128), 128, 0, b->stream>>>(
-            d_feats, m->sumlen, d_featoff, b->d_uttoff, n_utt, m->d_rec, m->d_rec_off, b->d_topn, b->d_tc_flags, (long long)fw, m->K,
-            m->n_feat, m->n_density);
-    else {
-        const unsigned blocks = (unsigned)((chains * 32 + 127) / 128);
+    const unsigned blocks = (unsigned)((chains * 32 + 127) / 128);
 #define PSB_FIXW(NDW) ptm_fixup_warp_kernel<13, NDW><<<blocks, 128, 0, b->stream>>>(d_feats, m->sumlen, d_featoff, b->d_uttoff, n_utt, \
-            m->d_rec, m->d_rec_off, b->d_topn, b->d_tc_flags, (long long)fw, m->K, m->n_feat)
-        if (m->n_density == 256) PSB_FIXW(8);
-        else if (m->n_density == 128) PSB_FIXW(4);
-        else PSB_FIXW(2);
+        m->d_rec, m->d_rec_off, b->d_topn, b->d_tc_flags, (long long)fw, m->K, m->n_feat)
+    if (m->n_density == 256) PSB_FIXW(8);
+    else if (m->n_density == 128) PSB_FIXW(4);
+    else PSB_FIXW(2);
 #undef PSB_FIXW
-    }
     PSB_LAUNCH_CHECK();
     return PSB_OK;
 }

@@ -359,33 +359,60 @@ def test_phoneloop_large_and_5state_vs_oracle(api, n_emit, H, window, skip):
 
 
 # ---------------------------------------------------------------------------------------
-# every top-N kernel variant (PSB_TOPN_VARIANT, read at psb_batch_create) must give the same bits
+# the scan kernels (PSB_TOPN_VARIANT=5, read at psb_batch_create) and the default selection by model shape (6) must
+# give the same bits; the last four models reach the fallbacks that only a model's shape selects
 
-@pytest.mark.parametrize("variant", [0, 1, 2, 3, 4, 5, 6])
-def test_topn_kernel_variants(api, en_us_dev, variant, monkeypatch):
-    from oracle import oracle
-    from pocketsphinx_b200.model import quantize_for_ties, synth_feats, synth_ptm
-    monkeypatch.setenv("PSB_TOPN_VARIANT", str(variant))
-    # (1) shipped model, real features
-    g = golden("en_us_goforward.npz")
-    b = api.Batch(en_us_dev, 4, 1024)
-    assert np.array_equal(b.score_host(g["feats"], np.array([0, 278], np.int32)), g["senscr"])
-    b.close()
-    # (2) BASELINE shape, ragged batch of 70 utterances (3 lane groups: an odd group count, padding
-    #     lanes, zero-length utterances)
-    pm = synth_ptm(seed=11, n_density=256, n_sen=600)
-    rng = np.random.default_rng(4)
-    lens = [0, 1, 40, 0, 17] + [int(x) for x in rng.integers(1, 40, 65)]
-    feats = synth_feats(pm, len(lens), 40, seed=3)
-    _batch_vs_oracle(api, pm, [feats[u][:n].reshape(n, pm.sumlen) for u, n in enumerate(lens)])
-    # (3) exact ties everywhere
-    pmq, gen = quantize_for_ties(synth_ptm(seed=2, n_density=64, n_sen=400), seed=6)
-    _batch_vs_oracle(api, pmq, list(gen(40, 25, s=9)))
-    # (4) frame down-sampling (-ds 2): odd frames only re-score the listed codewords
-    pm2 = synth_ptm(seed=12, n_density=128, n_sen=300)
-    pm2.ds_ratio = 2
-    f2 = synth_feats(pm2, 33, 20, seed=5)
-    _batch_vs_oracle(api, pm2, [f2[u].reshape(-1, pm2.sumlen) for u in range(33)])
+@pytest.mark.parametrize("case", ["en_us", "ragged", "ties", "ds2", "ptm_logbase", "semi_logbase", "semi_nd32", "ptm_fl39"])
+def test_topn_kernel_variants(api, en_us_dev, case, monkeypatch):
+    from pocketsphinx_b200.model import make_logadd8, quantize_for_ties, synth_feats, synth_ptm, synth_semi
+    if case == "ragged":
+        # BASELINE shape, ragged batch of 70 utterances (3 lane groups: an odd group count, padding lanes,
+        # zero-length utterances)
+        pm = synth_ptm(seed=11, n_density=256, n_sen=600)
+        lens = [0, 1, 40, 0, 17] + [int(x) for x in np.random.default_rng(4).integers(1, 40, 65)]
+        feats = synth_feats(pm, len(lens), 40, seed=3)
+        chunks = [feats[u][:n].reshape(n, pm.sumlen) for u, n in enumerate(lens)]
+    elif case == "ties":
+        # exact ties everywhere
+        pm, gen = quantize_for_ties(synth_ptm(seed=2, n_density=64, n_sen=400), seed=6)
+        chunks = list(gen(40, 25, s=9))
+    elif case == "ds2":
+        # frame down-sampling (-ds 2): odd frames only re-score the listed codewords
+        pm = synth_ptm(seed=12, n_density=128, n_sen=300)
+        pm.ds_ratio = 2
+        chunks = list(synth_feats(pm, 33, 20, seed=5))
+    elif case in ("ptm_logbase", "semi_logbase"):
+        # -logbase 1.00003: the add table's largest entry is 23 and 3 * 23 >= SEN_BIAS, so the senone stage takes
+        # ptm_senone_kernel<false> / semi_senone_kernel<false> instead of the 16x2 kernels
+        pm = (synth_ptm if case == "ptm_logbase" else synth_semi)(seed=31, n_density=64, n_sen=400)
+        pm.logadd8 = make_logadd8(base=1.00003)
+        chunks = list(synth_feats(pm, 20, 25, seed=4))
+    elif case == "semi_nd32":
+        # semi-continuous with n_density 32, outside the split path: ptm_topn2_kernel for the 12- and 3-dimensional
+        # streams, the float scalar ptm_topn_kernel<24, true, false> for the 24-dimensional one
+        pm = synth_semi(seed=32, n_density=32, n_sen=300)
+        chunks = list(synth_feats(pm, 20, 25, seed=4))
+    elif case == "ptm_fl39":
+        # PTM with one 39-dimensional stream (no tensor-core filter): the float scalar ptm_topn_kernel<39, false, false>
+        pm = synth_ptm(seed=33, n_feat=1, featlen=39, n_density=64, n_sen=400)
+        chunks = list(synth_feats(pm, 20, 25, seed=4))
+    for variant in (5, 6):
+        monkeypatch.setenv("PSB_TOPN_VARIANT", str(variant))
+        if case == "en_us":
+            # shipped model, real features
+            g = golden("en_us_goforward.npz")
+            b = api.Batch(en_us_dev, 4, 1024)
+            assert np.array_equal(b.score_host(g["feats"], np.array([0, 278], np.int32)), g["senscr"]), variant
+            b.close()
+        else:
+            _batch_vs_oracle(api, pm, chunks)
+
+
+def test_topn_variant_outside_the_accepted_values_is_refused(api, en_us_dev, monkeypatch):
+    """Values of PSB_TOPN_VARIANT that once selected other kernels are refused, not silently mapped to a path."""
+    monkeypatch.setenv("PSB_TOPN_VARIANT", "2")
+    with pytest.raises(api.PsbError, match="accepted: 5"):
+        api.Batch(en_us_dev, 4, 1024)
 
 
 TC_CHECK = r"""
@@ -417,20 +444,18 @@ print(json.dumps(out))
 """
 
 
-@pytest.mark.parametrize("impl", ["tcgen05", "mma"])
-def test_tensor_core_filter_error_bound_holds_on_the_device(impl):
+def test_tensor_core_filter_error_bound_holds_on_the_device():
     """PSB_TC_CHECK=1: the filter kernel compares every 3 x TF32 GEMM value it produced with the exact float
     distance and reports the worst |a - d| / eps (the bound the candidate selection relies on must hold
     with room to spare: the analysis in psb_ptm_tc.cu allows 0.8 of eps), on the shipped model with real
-    features, the BASELINE shape, features scaled far outside the model's range and tie-stress data; for the
-    tcgen05 / tensor-memory kernel (the default) and for the legacy mma.sync variant (PSB_TC_IMPL=mma)."""
+    features, the BASELINE shape, features scaled far outside the model's range and tie-stress data."""
     import json
     import os
     import subprocess
     import sys
     from conftest import GOLDEN, ROOT
     code = TC_CHECK % (ROOT, os.path.join(ROOT, "tests"), os.path.join(GOLDEN, "en_us_ptm_model.npz"))
-    r = subprocess.run([sys.executable, "-c", code], env=dict(os.environ, PSB_TC_CHECK="1", PSB_TOPN_VARIANT="6", PSB_TC_IMPL=impl),
+    r = subprocess.run([sys.executable, "-c", code], env=dict(os.environ, PSB_TC_CHECK="1", PSB_TOPN_VARIANT="6"),
                        capture_output=True, text=True, timeout=900)
     assert r.returncode == 0, r.stderr[-3000:]
     out = json.loads(r.stdout.strip().splitlines()[-1])
@@ -665,8 +690,8 @@ def test_full_size_properties(api, monkeypatch):
     om = oracle.OracleModel(pm)
     for u, got in sample5.items():
         assert np.array_equal(got, om.score_utt(feats[u])), "utterance %d" % u
-    # same bits from the packed kernel without deferred insertion, and from two ranges in flight
-    best2, pen2, rows2, _, _ = run(2, 2)
+    # same bits from two ranges in flight
+    best2, pen2, rows2, _, _ = run(5, 2)
     assert np.array_equal(rows5, rows2)
     assert np.array_equal(best5, best2) and np.array_equal(pen5, pen2)
     # and from the path without the recurrence over time (tensor-core filter + exact rescoring + tie fix-up)
